@@ -6,7 +6,7 @@ A "step" = one forward of BASELINE config 2 per GPU: 1 synthetic Waymo-shaped sw
 layers, d=128, h=8, ff=256), sparse output (to_bev=False, no attached convs).  Frames shard over GPUs
 (weak scaling, no data-path collective: inference has none, SURVEY.md 8e).
 
-    python bench.py --gpus 1 --steps 20 --warmup 5
+    python bench.py --gpus 1 --steps 600 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # CPU port of the reference path on the host cores
 """
@@ -27,6 +27,8 @@ P_POINTS = 150000
 METRIC = "lidar_frames_per_sec_sst6_fwd_150k"
 # one workload string for both arms (the driver compares them)
 WORKLOAD = "config2: SST-6 fwd, 150k-pt Waymo-shaped sweep, 0.32m pillars, d=128 h=8 ff=256, batch 1 per GPU, sparse output"
+DUMP_MAX_ROWS = 100000
+WINDOW_STEPS = 20   # steps per timed window: long enough to keep every engine stream busy, short enough to give many windows
 
 
 def ncu_layer_traffic():
@@ -146,6 +148,25 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm), "source": f"{self.mode}, samples {where}"}
+
+
+def dump_outputs(out_dir, feats, coors, num):
+    """What a caller of the engine receives from one run(): the first `num` rows of the feature and coordinate buffers.
+    Coordinates are stored as float64 (exact for int32), so that every file is float32 or float64.  Above DUMP_MAX_ROWS rows
+    (64 MB in all at d = 128) a fixed seeded sample of rows is stored, with its row indices."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    M = int(num.item())
+    rows = torch.arange(M)
+    if M > DUMP_MAX_ROWS:
+        rows = torch.randperm(M, generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ROWS].sort().values
+    arrays = {"voxel_feats": feats[:M][rows.to(feats.device)].float().cpu().numpy(),
+              "voxel_coors": coors[:M][rows.to(coors.device)].cpu().numpy().astype(np.float64),
+              "num_voxels": np.array([M], dtype=np.float64)}
+    if M > DUMP_MAX_ROWS:
+        arrays["row_index"] = rows.numpy().astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 _BEST_THREADS = None
@@ -283,7 +304,7 @@ def train_bench(args, world, rank, dev, frames_d):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=600, help=f"timed steps (frames per GPU), in windows of {WINDOW_STEPS}")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default=os.environ.get("SSTB200_PRECISION", "auto"))
@@ -294,7 +315,11 @@ def main():
     ap.add_argument("--train-frames", type=int, default=4, help="frames per GPU and training step (config 4: 32 frames / 8 GPUs)")
     ap.add_argument("--streams", type=int, default=int(os.environ.get("SSTB200_STREAMS", "8")),
                     help="frames in flight per GPU (independent engines on their own CUDA streams); 1 = strictly serial")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (voxel features, voxel coordinates, voxel count) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -312,8 +337,10 @@ def main():
     all_cpus = os.sched_getaffinity(0)
     numa_cpus = pin_to_gpu_numa(local)   # host thread + pinned staging buffers on the GPU's NUMA node (None: topology not exposed)
 
-    from sst_b200 import build, flagship as fl
-    build.build()
+    from sst_b200 import _lib, build, flagship as fl
+    if build.needs_build():   # nothing is compiled or written here: a library older than its sources is an error, not a benchmark
+        raise SystemExit(f"{build.OUT} is missing or older than its sources: run `python -m sst_b200.build` first")
+    _lib.lib()
     from sst_b200.engine import SSTEngine
 
     cfg = fl.sst_cfg()
@@ -356,38 +383,43 @@ def main():
 
     sampler = ClockSampler(local)
     sampler.start()   # before the warm-up; samples are kept only inside the timed windows (begin/end)
-    for i in range(max(args.warmup, S)):
+    n_warm = max(args.warmup, S)
+    for i in range(n_warm):
         step(i)
     barrier()
     sampler.begin()
     main = torch.cuda.current_stream(dev)
-    REPS = int(os.environ.get("SSTB200_BENCH_REPS", "30"))   # the K-step window is repeated and the MEDIAN window reported
-    windows = []
     ncu_range = os.environ.get("SSTB200_NCU_RANGE") == "1"   # `ncu --profile-from-start off`: profile the first timed window only
-    for rep in range(REPS):
-        if ncu_range and rep == 0:
+    # exactly --steps timed steps, in consecutive windows of WINDOW_STEPS; the median window sets the value, the spread is reported.
+    # The timed steps start at the frame after the warm-up's, so none of them reads a sweep the warm-up just left in L2.
+    windows = []
+    for w0 in range(0, args.steps, WINDOW_STEPS):
+        n = min(WINDOW_STEPS, args.steps - w0)
+        if ncu_range and w0 == 0:
             torch.cuda.profiler.start()
-        if ncu_range and rep == 1:
-            torch.cuda.synchronize()
-            torch.cuda.profiler.stop()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(main)
         for e in engs:
             e.stream.wait_event(e0)
-        for i in range(args.steps):
-            step(rep * args.steps + i)
+        for i in range(w0, w0 + n):
+            last = step(n_warm + i)
         for e in engs:
             main.wait_stream(e.stream)
         e1.record(main)
-        windows.append((e0, e1))
+        windows.append((e0, e1, n))
+        if ncu_range and w0 == 0:
+            torch.cuda.synchronize()
+            torch.cuda.profiler.stop()
     barrier()
     sampler.end()
-    wms = torch.tensor([a.elapsed_time(b) for a, b in windows], dtype=torch.float64, device=dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    wms = torch.tensor([a.elapsed_time(b) for a, b, _ in windows], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(wms, op=dist.ReduceOp.MAX)   # per window: the slowest rank
-    wms = sorted(wms.tolist())
-    total_ms = wms[len(wms) // 2]
-    value = world * args.steps / (total_ms / 1e3)
+    ms_step = sorted(ms / n for ms, (_, _, n) in zip(wms.tolist(), windows))
+    ms_per_step = ms_step[len(ms_step) // 2]
+    value = world / (ms_per_step / 1e3)
 
     # serial single-stream latency per frame (CUDA events around each step, L2 flushed in between) - reported beside it
     flush = torch.empty(512 << 20, dtype=torch.uint8, device=dev)
@@ -552,7 +584,8 @@ def main():
     if rank == 0:
         line = {
             "metric": METRIC, "value": value, "unit": "frames/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
-            "ms_per_step": total_ms / args.steps, "windows": {"repeats": len(wms), "ms_min": wms[0], "ms_median": total_ms, "ms_max": wms[-1]},
+            "ms_per_step": ms_per_step, "windows": {"repeats": len(ms_step), "steps_per_window": WINDOW_STEPS, "ms_per_step_min": ms_step[0],
+                                                    "ms_per_step_median": ms_per_step, "ms_per_step_max": ms_step[-1]},
             "latency_ms_single_stream": latency_ms, "value_one_frame_in_flight": world * 1e3 / latency_ms,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32" if precision == "fp32" else "f16", "data": "synthetic",

@@ -9,6 +9,7 @@ tests/test_oracle_golden.py can pin oracle/sst_oracle.py against them anywhere (
 dynamic_point_to_voxel, voxelization.h:96-108); that op is pinned separately (restated reference test +
 reference CUDA build in oracle/_ref on GPU boxes).
 """
+import json
 import os
 import sys
 
@@ -431,8 +432,401 @@ def fsd_cluster_fixture():
     print("fsd_cluster", {k: int(out[k].max()) + 1 for k in out if k.startswith("cc_labels_")})
 
 
+# ---- reference pins: what tests/test_oracle_*_vs_reference.py, test_ref_voxel_layer.py and test_host_logic.py compare with ----------
+# Stored as compact records (oracle/golden_io.py): digests where the tests demand bit equality, seeded row samples + projections where
+# they allow a tolerance.  Weights are regenerated from seeds on both sides (golden_io.seeded_state), inputs by the functions below.
+SST_VS = VS
+PIN_DROP_TEST = DROP_TEST
+
+
+def pin_dsvfe_points():
+    g = torch.Generator().manual_seed(17)
+    vs, rng = (0.25, 0.25, 0.2), [-80, -80, -2, 80, 80, 4]
+    pts = torch.cat([torch.cat([O.synth_frame(3 + b, 3000), torch.rand(3000, 2, generator=g)], 1) for b in range(2)])
+    co = torch.cat([torch.nn.functional.pad(O.dynamic_voxelize(pts[b * 3000:(b + 1) * 3000], vs, rng), (1, 0), value=b)
+                    for b in range(2)]).long()
+    return pts, co, vs, rng
+
+
+def pin_neck_inputs():
+    g = torch.Generator().manual_seed(5)
+    N, M, C = 5000, 700, 16
+    pts = O.synth_frame(3, N, extra_dims=1)
+    coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0).long()
+    vf = torch.randn(M, C, generator=g)
+    vf[::7] = -1.0  # dropped voxels are padded rows
+    inds = torch.randint(0, M, (N,), generator=g)
+    return pts, coors, vf, inds
+
+
+def pin_sir_inputs():
+    N, G = 3000, 40
+    g = torch.Generator().manual_seed(2)
+    points = torch.cat([torch.randn(N, 3, generator=g) * 10, torch.rand(N, 2, generator=g)], 1)
+    feats = torch.randn(N, 27, generator=g)
+    gid = torch.randint(0, G, (N,), generator=g)
+    coors = torch.stack([gid % 3, torch.zeros_like(gid), gid], 1)
+    fcl = torch.randn(N, 3, generator=g) * 2
+    return points, feats, coors, fcl
+
+
+def sst_pins_fixture(R):
+    from oracle import golden_io as GI
+    out = {}
+    vfe_kw = dict(in_channels=3, with_cluster_center=True, with_voxel_center=True, voxel_size=VS, point_cloud_range=RNG,
+                  norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01))
+    bb_kw = dict(d_model=[64], nhead=[4], num_blocks=1, dim_feedforward=[128], output_shape=[468, 468], num_attached_conv=0, to_bev=False)
+    # config 1: 20k points, DynamicVFE -> SSTInputLayerV2 -> one SSTv2 block
+    pts = O.synth_frame(1000, 20000)
+    coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0)
+    vfe = R.DynamicVFE(feat_channels=[64, 64], **vfe_kw).eval()
+    il = R.SSTInputLayerV2(DROP_TEST, (12, 12, 1), (468, 468, 1), shuffle_voxels=False, debug=True, mute=True).eval()
+    bb = R.SSTv2(**bb_kw).eval()
+    out["config1.vfe_spec"], out["config1.bb_spec"] = GI.state_spec(vfe), GI.state_spec(bb)
+    GI.load_seeded(vfe, out["config1.vfe_spec"], 101)
+    GI.load_seeded(bb, out["config1.bb_spec"], 102)
+    with torch.no_grad():
+        vf_r, vc_r = vfe(pts, coors)
+        info_r = il(vf_r, vc_r, 1)
+        out_r = bb(info_r)[0]["voxel_feats"]
+    GI.record(out, "config1.vc", vc_r, exact=True)
+    GI.record(out, "config1.vf", vf_r)
+    for i in range(2):
+        for k in (f"batch_win_inds_shift{i}", f"coors_in_win_shift{i}", f"voxel_drop_level_shift{i}"):
+            GI.record(out, f"config1.{k}", info_r[k], exact=True)
+    GI.record(out, "config1.out", out_r)
+    # state-dict keys and shapes of the reference classes
+    from sst_b200 import flagship as fl
+    cfg = fl.sst_cfg(num_blocks=2)
+    r_vfe = R.DynamicVFE(**{k: v for k, v in cfg['voxel_encoder'].items() if k != 'type'})
+    r_bb = R.SSTv2(**{k: v for k, v in cfg['backbone'].items() if k != 'type'})
+    lc = dict(cosine=True, non_shared_tau=True, use_bn=True)
+    r_cos = R.SSTv2(d_model=[32], nhead=[4], num_blocks=1, dim_feedforward=[64], num_attached_conv=0, to_bev=False, layer_cfg=lc)
+    for name, m in (("vfe", r_vfe), ("bb", r_bb), ("cosine", r_cos)):
+        out[f"keys.{name}"] = {k: list(v.shape) for k, v in m.state_dict().items()}
+    # Voxel2PointScatterNeck
+    pts_n, coors_n, vf_n, inds_n = pin_neck_inputs()
+    for with_xyz, norm in ((True, False), (True, True), (False, False)):
+        neck = R.Voxel2PointScatterNeck(point_cloud_range=RNG, voxel_size=VS, with_xyz=with_xyz, normalize_local_xyz=norm).eval()
+        r_out, r_mask = neck(pts_n, coors_n, vf_n, inds_n)
+        GI.record(out, f"neck.{with_xyz}.{norm}.out", r_out, exact=True)
+        GI.record(out, f"neck.{with_xyz}.{norm}.mask", r_mask, exact=True)
+    # gradients of DynamicVFE -> SSTInputLayerV2 -> SSTv2 (eval-mode BN, one block)
+    pts = O.synth_frame(1000, 6000)
+    coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0)
+    vfe = R.DynamicVFE(feat_channels=[32, 64], **vfe_kw).eval()
+    bb = R.SSTv2(**bb_kw).eval()
+    out["grad.vfe_spec"], out["grad.bb_spec"] = GI.state_spec(vfe), GI.state_spec(bb)
+    GI.load_seeded(vfe, out["grad.vfe_spec"], 103)
+    GI.load_seeded(bb, out["grad.bb_spec"], 104)
+    p_r = pts.clone().requires_grad_(True)
+    vf_r, vc_r = vfe(p_r, coors)
+    out_r = bb(il(vf_r, vc_r, 1))[0]["voxel_feats"]
+    out_r.square().mean().backward()
+    GI.record(out, "grad.points", p_r.grad)
+    for pre, m in (("vfe.", vfe), ("bb.", bb)):
+        for k, v in m.named_parameters():
+            GI.record(out, "grad." + pre + k, v.grad, rows=4)
+    # SIR gradients
+    m = R.SIR(num_blocks=2, in_channels=[32, 37], feat_channels=[[32, 32], [32, 32]], rel_mlp_hidden_dims=[[16, 32], [16, 32]],
+              norm_cfg=dict(type='LN', eps=1e-3), mode='max', xyz_normalizer=[20, 20, 4], act='gelu', unique_once=True).eval()
+    out["sir.spec"] = GI.state_spec(m)
+    GI.load_seeded(m, out["sir.spec"], 105)
+    points, feats, coors_s, fcl = pin_sir_inputs()
+    f_r = feats.clone().requires_grad_(True)
+    a, b, _ = m(points, f_r, coors_s, fcl)
+    (a.square().mean() + b.square().mean()).backward()
+    GI.record(out, "sir.feats", f_r.grad)
+    for k, p in m.named_parameters():
+        GI.record(out, "sir." + k, p.grad, rows=4)
+    # DynamicVFE in train(): outputs, gradients, running buffers after the step
+    vfe = R.DynamicVFE(feat_channels=[32, 64], **vfe_kw).train()
+    out["train.spec"] = GI.state_spec(vfe)
+    GI.load_seeded(vfe, out["train.spec"], 106)
+    p_r = pts.clone().requires_grad_(True)
+    vf_r, vc_r = vfe(p_r, coors)
+    vf_r.square().mean().backward()
+    GI.record(out, "train.vc", vc_r, exact=True)
+    GI.record(out, "train.vf", vf_r)
+    GI.record(out, "train.points", p_r.grad)
+    for k, p in vfe.named_parameters():
+        GI.record(out, "train." + k, p.grad, rows=4)
+    sd = vfe.state_dict()
+    for k in ("vfe_layers.0.norm.running_mean", "vfe_layers.0.norm.running_var"):
+        GI.record(out, "train." + k, sd[k])
+    # DynamicScatterVFE in train()
+    pts_d, co_d, vs, rng = pin_dsvfe_points()
+    m = R.DynamicScatterVFE(in_channels=5, feat_channels=[32, 32], with_cluster_center=True, with_voxel_center=True, voxel_size=vs,
+                            point_cloud_range=rng, norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01), unique_once=True,
+                            rel_dist_scaler=10.0).train()
+    out["dsvfe.spec"] = GI.state_spec(m)
+    GI.load_seeded(m, out["dsvfe.spec"], 107)
+    x = pts_d.clone().requires_grad_(True)
+    vf, vc, inv = m(x, co_d, return_inv=True)
+    probe = torch.randn(vf.shape, generator=torch.Generator().manual_seed(1))
+    (vf * probe).sum().backward()
+    GI.record(out, "dsvfe.vc", vc, exact=True)
+    GI.record(out, "dsvfe.inv", inv, exact=True)
+    GI.record(out, "dsvfe.vf", vf)
+    GI.record(out, "dsvfe.points", x.grad)
+    for k, p in m.named_parameters():
+        GI.record(out, "dsvfe." + k, p.grad, rows=4)
+    GI.save(os.path.join(OUT, "ref_sst_pins.npz"), out)
+    print("ref_sst_pins", len(out), "arrays")
+
+
+def fsd_pins_fixture():
+    from oracle import fsd_oracle as FO, golden_io as GI
+    RF = ref_shim.reference_functions("mmdet3d/models/detectors/single_stage_fsd.py",
+                                      ["filter_almost_empty", "find_connected_componets", "find_connected_componets_single_batch",
+                                       "modify_cluster_by_class", "ClusterAssigner"])
+    out = {}
+    pts, bidx = FO.synth_centres(3, 3, 700)
+    for d in (0.1, 0.6, 2.0):
+        GI.record(out, f"cc.{d}", RF["find_connected_componets"](pts, bidx, d), exact=True)
+        GI.record(out, f"cc_single.{d}", RF["find_connected_componets_single_batch"](pts[:700], bidx[:700], d), exact=True)
+    ca = RF["ClusterAssigner"](**FSD_CA_CFG)
+    ca.num_classes = 3
+    ca.train()
+    pts_l, b_l = pin_cluster_inputs()
+    inds, masks = ca(pts_l, b_l, origin_points=[None] * 3)
+    for i in range(3):
+        GI.record(out, f"ca.class{i}", inds[i][:, 0].long(), exact=True)
+        GI.record(out, f"ca.inds{i}", inds[i][:, 1:].int(), exact=True)
+        GI.record(out, f"ca.mask{i}", masks[i], exact=True)
+    ca.eval()
+    m0 = b_l[0] == 0
+    inds1, _ = ca([pts_l[0][m0]], [b_l[0][m0]], origin_points=[None])
+    GI.record(out, "ca.eval_inds", inds1[0][:, 1:].int(), exact=True)
+    GI.save(os.path.join(OUT, "ref_fsd_pins.npz"), out)
+    print("ref_fsd_pins", len(out), "arrays")
+
+
+FSD_CA_CFG = dict(cluster_voxel_size=dict(Car=(0.3, 0.3, 6), Cyclist=(0.2, 0.2, 6), Pedestrian=(0.05, 0.05, 6)), min_points=2,
+                  point_cloud_range=[-80, -80, -2, 80, 80, 4], connected_dist=dict(Car=0.6, Cyclist=0.4, Pedestrian=0.1),
+                  class_names=['Car', 'Cyclist', 'Pedestrian'])
+
+
+def pin_cluster_inputs():
+    from oracle import fsd_oracle as FO
+    pts_l, b_l = [], []
+    for i, blob in enumerate((0.5, 0.3, 0.08)):
+        p, b = FO.synth_centres(10 + i, 2, 1500, blob=blob)
+        order = torch.argsort(b, stable=True)
+        pts_l.append(p[order])
+        b_l.append(b[order])
+    return pts_l, b_l
+
+
+SPCONV_PIN_CONV = [(3, 2, 1), (3, 2, (0, 1, 1)), ((3, 1, 1), (2, 1, 1), 0), (2, 2, 0)]
+SPCONV_PIN_SUBM = [(3, 1), ((3, 1, 1), (1, 0, 0)), (3, 0), (3, (0, 1, 1))]
+SPCONV_PIN_UNET = dict(in_channels=8, sparse_shape=[9, 32, 32], order=('conv', 'norm', 'act'),
+                       norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01), base_channels=8, output_channels=16,
+                       encoder_channels=((8,), (8, 8, 8), (16, 16, 16), (16, 16, 16)),
+                       encoder_paddings=((1,), (1, 1, 1), (1, 1, 1), ((0, 1, 1), 1, 1)),
+                       decoder_channels=((16, 16, 16), (16, 16, 8), (8, 8, 8), (8, 8, 8)), decoder_paddings=((1, 1), (1, 0), (0, 0), (0, 1)))
+SPCONV_PIN_MIXER = dict(in_channels=8, sparse_shape=[8, 24, 24], norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01), base_channels=8,
+                        output_channels=12, encoder_channels=((8,), (8, 8), (8, 8)), encoder_paddings=((1,), (1, 1), (1, 1)),
+                        decoder_channels=((8, 8, 8), (8, 8, 8), (8, 8, 8)), decoder_paddings=((1, 1), (1, 1), (1, 1)))
+
+
+def spconv_pins_fixture():
+    """The reference's vendored spconv v1 layers and sparse U-Nets with seeded weights (rows of strided outputs sorted by coordinate)."""
+    from oracle import golden_io as GI, spconv_oracle as SO
+    S = ref_shim.load_spconv()
+    out = {}
+    feats, coors = SO.synth_sparse(1, 2, (9, 20, 24), 300, 8)
+    for i, (ks, stride, padding) in enumerate(SPCONV_PIN_CONV):
+        conv = S.SparseConv3d(8, 12, ks, stride=stride, padding=padding, bias=False, indice_key="k")
+        inv = S.SparseInverseConv3d(12, 6, ks, indice_key="k", bias=False)
+        GI.load_seeded(conv, GI.state_spec(conv), 200 + i)
+        GI.load_seeded(inv, GI.state_spec(inv), 210 + i)
+        with torch.no_grad():
+            y = conv(S.SparseConvTensor(feats, coors, [9, 20, 24], 2))
+            z = inv(y)
+        yf, yc = _sort_rows(y.features, y.indices)
+        out[f"conv{i}.geometry"] = [list(conv.kernel_size), list(conv.stride), list(conv.padding)]
+        out[f"conv{i}.spatial_shape"] = [int(v) for v in y.spatial_shape]
+        GI.record(out, f"conv{i}.coors", yc.int(), exact=True)
+        GI.record(out, f"conv{i}.out", yf, rows=GI.MIN_ROWS)
+        GI.record(out, f"conv{i}.inv_coors", z.indices, exact=True)
+        GI.record(out, f"conv{i}.inv_out", z.features, rows=GI.MIN_ROWS)
+    feats, coors = SO.synth_sparse(2, 2, (7, 18, 18), 250, 8)
+    for i, (ks, padding) in enumerate(SPCONV_PIN_SUBM):
+        conv = S.SubMConv3d(8, 10, ks, padding=padding, bias=True, indice_key="s")
+        GI.load_seeded(conv, GI.state_spec(conv), 220 + i)
+        with torch.no_grad():
+            y = conv(S.SparseConvTensor(feats, coors, [7, 18, 18], 2))
+        out[f"subm{i}.kernel_size"] = list(conv.kernel_size)
+        GI.record(out, f"subm{i}.coors", y.indices, exact=True)
+        GI.record(out, f"subm{i}.out", y.features, rows=GI.MIN_ROWS)
+    net = S.SimpleSparseUNet(**SPCONV_PIN_UNET, return_multiscale_features=True).eval()
+    out["unet.spec"] = GI.state_spec(net)
+    GI.load_seeded(net, out["unet.spec"], 230)
+    feats, coors = SO.synth_sparse(4, 2, (9, 32, 32), 500, 8)
+    with torch.no_grad():
+        r = net(dict(voxel_feats=feats, voxel_coors=coors))[0]
+    GI.record(out, "unet.coors", r["voxel_coors"], exact=True)
+    GI.record(out, "unet.out", r["voxel_feats"], rows=GI.MIN_ROWS)
+    out["unet.n_levels"] = len(r["decoder_features"])
+    for i, d in enumerate(r["decoder_features"]):
+        f, c = _sort_rows(d.features, d.indices)
+        GI.record(out, f"unet.ms{i}.coors", c.int(), exact=True)
+        GI.record(out, f"unet.ms{i}.out", f, rows=GI.MIN_ROWS)
+    net = S.VirtualVoxelMixer(**SPCONV_PIN_MIXER).eval()
+    out["mixer.spec"] = GI.state_spec(net)
+    GI.load_seeded(net, out["mixer.spec"], 240)
+    feats, coors = SO.synth_sparse(8, 3, (8, 24, 24), 300, 8)
+    with torch.no_grad():
+        rf, rc, rshape = net(feats, coors, 3)
+    GI.record(out, "mixer.coors", rc, exact=True)
+    out["mixer.spatial_shape"] = [int(v) for v in rshape]
+    GI.record(out, "mixer.out", rf, rows=GI.MIN_ROWS)
+    GI.save(os.path.join(OUT, "ref_spconv_pins.npz"), out)
+    print("ref_spconv_pins", len(out), "arrays")
+
+
+VOXEL_PIN_CASES = [(VS, RNG), ((0.25, 0.25, 0.2), [-80, -80, -2, 80, 80, 4]), ((0.1, 0.1, 0.15), [-51.2, -51.2, -5, 51.2, 51.2, 3])]
+HV_PIN_CASES = [  # (P, F, voxel_size, range, max_points, max_voxels)
+    (20000, 4, (0.32, 0.32, 6), [-74.88, -74.88, -2, 74.88, 74.88, 4], 32, 20000),
+    (20000, 4, (0.32, 0.32, 6), [-74.88, -74.88, -2, 74.88, 74.88, 4], 5, 300),       # both caps bite
+    (30000, 5, (0.5, 0.5, 0.25), [-40, -40, -3, 40, 40, 1], 10, 16000),               # 3-D grid
+    (7, 3, (1.0, 1.0, 1.0), [0, 0, 0, 4, 4, 4], 2, 3),
+    (150000, 4, (0.32, 0.32, 6), [-74.88, -74.88, -2, 74.88, 74.88, 4], 32, 32000),
+]
+
+
+def pin_voxel_points():
+    pts = O.synth_frame(11, 40000)
+    pts[::7, 0] += 200.0
+    pts[::11, 1] -= 300.0
+    return pts
+
+
+def pin_hv_points(P, F):
+    pts = O.synth_frame(300 + P, P, extra_dims=F - 3)
+    pts[::13, 0] += 500.0  # out of range -> clamped by this fork's voxeliser
+    return pts
+
+
+def voxel_layer_pins_fixture():
+    """The reference's own C++ dynamic_voxelize / hard_voxelize (voxelization_cpu.cpp, compiled unmodified into oracle/_ref)."""
+    from oracle import build_ref, golden_io as GI
+    ref = build_ref.load_module() or (build_ref.build() and build_ref.load_module())
+    out = {}
+    pts = pin_voxel_points()
+    for i, (vs, rng) in enumerate(VOXEL_PIN_CASES):
+        co = torch.zeros((pts.shape[0], 3), dtype=torch.int32)
+        ref.dynamic_voxelize(pts, co, list(vs), list(rng), 3)
+        GI.record(out, f"dyn{i}.coors", co, exact=True)
+    for i, (P, F, vs, rng, mp, mv) in enumerate(HV_PIN_CASES):
+        pts = pin_hv_points(P, F)
+        voxels = torch.zeros((mv, mp, F))
+        coors = torch.zeros((mv, 3), dtype=torch.int32)
+        npts = torch.zeros((mv,), dtype=torch.int32)
+        n = ref.hard_voxelize(pts, voxels, coors, npts, list(vs), list(rng), mp, mv, 3)
+        out[f"hv{i}.n"] = int(n)
+        GI.record(out, f"hv{i}.voxels", voxels[:n], exact=True)
+        GI.record(out, f"hv{i}.coors", coors[:n], exact=True)
+        GI.record(out, f"hv{i}.npts", npts[:n], exact=True)
+    GI.save(os.path.join(OUT, "ref_voxel_layer_pins.npz"), out)
+    print("ref_voxel_layer_pins", len(out), "arrays")
+
+
+SCATTER_PIN_CASES = [(150000, 128, 0), (200000, 3, -1), (5000, 64, -1), (17, 5, 0)]
+VOXEL_CUDA_PIN_SIZES = [1, 20000, 150000]
+
+
+def pin_scatter_inputs(P, C, lo):
+    """feats, coors and output-gradient generator of one dynamic-scatter case (CPU tensors; for the sweep-sized cases the coors come from
+    the oracle's voxeliser, oracle.sst_oracle.dynamic_voxelize, so that they do not depend on the implementation under test)."""
+    g = torch.Generator().manual_seed(P + C)
+    feats = torch.rand(P, C, generator=g) * 100 - 50
+    if P >= 100000:
+        pts = O.synth_frame(5, P)
+        coors = O.dynamic_voxelize(pts, VS, RNG)
+    else:
+        coors = torch.randint(lo, 20, (P, 3), generator=g, dtype=torch.int32)
+    return feats, coors, g
+
+
+def pin_voxel_cuda_points(P):
+    pts = O.synth_frame(77 + P, P)
+    pts[::5, 0] += 300.0
+    return pts
+
+
+def ref_cuda_pins_fixture(out_dir=OUT):
+    """The reference's own CUDA dynamic_voxelize and dynamic_point_to_voxel_forward / backward (voxelization_cuda.cu,
+    scatter_points_cuda.cu, compiled unmodified into oracle/_ref) on a GPU: `python -m oracle.make_golden cuda-pins [DIR]`."""
+    from oracle import build_ref, golden_io as GI
+    ref = build_ref.load_module()
+    assert ref is not None, "oracle/_ref/voxel_layer_ref*.so not built"
+    dev = torch.device("cuda:0")
+    out = {}
+    for P in VOXEL_CUDA_PIN_SIZES:
+        pts = pin_voxel_cuda_points(P).to(dev)
+        r = torch.zeros((P, 3), dtype=torch.int32, device=dev)
+        ref.dynamic_voxelize(pts, r, list(VS), list(RNG), 3)
+        GI.record(out, f"voxelize{P}", r, exact=True)
+    for reduce in ("max", "mean", "sum"):
+        for P, C, lo in SCATTER_PIN_CASES:
+            feats, coors, g = pin_scatter_inputs(P, C, lo)
+            feats, coors = feats.to(dev), coors.to(dev)
+            r_f, r_c, r_m, r_n = ref.dynamic_point_to_voxel_forward(feats, coors, reduce)
+            key = f"scatter.{reduce}.{P}.{C}"
+            GI.record(out, key + ".coors", r_c, exact=True)
+            GI.record(out, key + ".map", r_m, exact=True)
+            GI.record(out, key + ".count", r_n, exact=True)
+            GI.record(out, key + ".feats", r_f, exact=reduce == "max")
+            grad = torch.randn(r_f.shape, generator=g).to(dev)
+            r_g = torch.zeros_like(feats)
+            ref.dynamic_point_to_voxel_backward(r_g, grad, feats, r_f, r_m, r_n, reduce)
+            GI.record(out, key + ".grad", r_g)
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    GI.save(os.path.join(out_dir, "ref_cuda_pins.npz"), out)
+    print("ref_cuda_pins", len(out), "arrays")
+
+
+REF_CONFIG_DIRS = ("configs/sst", "configs/sst_refactor", "configs/fsd", "configs/fsdv2")
+
+
+def reference_configs_fixture():
+    """The `model` dict of every config under configs/sst (v1 names), configs/sst_refactor, configs/fsd and configs/fsdv2, as parsed by the
+    stand-in Config loader (inheritance resolved), written as Python literals."""
+    import glob
+    from sst_b200.config import Config
+    files = sorted(f for d in REF_CONFIG_DIRS for f in glob.glob(os.path.join(ref_shim.REF_ROOT, d, "*.py")))
+    # configs/sst/to_be_done_do_not_use.py inherits from a _base_ file that does not exist in the reference tree: mmcv cannot load it either
+    files = [f for f in files if not f.endswith("to_be_done_do_not_use.py")]
+    models = {os.path.relpath(f, ref_shim.REF_ROOT): _plain(Config.fromfile(f).get("model", {})) for f in files}
+    names = sorted(models)
+    np.savez_compressed(os.path.join(OUT, "reference_configs.npz"), files=np.array(names), models=np.array([repr(models[k]) for k in names]))
+    print("reference_configs", len(models), "files")
+
+
+def _plain(v):
+    if isinstance(v, dict):
+        return {k: _plain(x) for k, x in v.items()}
+    if isinstance(v, (list, tuple)):
+        return type(v)(_plain(x) for x in v)
+    return v
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
+    if "cuda-pins" in sys.argv[1:]:   # on a GPU machine that has oracle/_ref
+        args = [a for a in sys.argv[1:] if a != "cuda-pins"]
+        ref_cuda_pins_fixture(args[0] if args else OUT)
+        sys.exit(0)
+    if "pins" in sys.argv[1:]:   # only the reference pins
+        sst_pins_fixture(ref_shim.load())
+        fsd_pins_fixture()
+        spconv_pins_fixture()
+        voxel_layer_pins_fixture()
+        reference_configs_fixture()
+        sys.exit(0)
     if "fsdv2" in sys.argv[1:]:
         fsdv2_front_fixture(ref_shim.load())
         sys.exit(0)
@@ -454,3 +848,8 @@ if __name__ == "__main__":
     hard_voxelize_fixture()
     spconv_fixture()
     fsd_cluster_fixture()
+    sst_pins_fixture(R)
+    fsd_pins_fixture()
+    spconv_pins_fixture()
+    voxel_layer_pins_fixture()
+    reference_configs_fixture()

@@ -1,14 +1,11 @@
-"""CPU: host-side logic of the package (no GPU, no compute calls): registry/config loading of the reference's own
-config files, positional table vs the oracle, drop-possibility check, lazy reference-layout dicts."""
-import glob
+"""CPU: host-side logic of the package (no GPU, no compute calls): registry builds from the reference's own config dicts,
+positional table vs the oracle, drop-possibility check, lazy reference-layout dicts."""
 import os
 
 import pytest
 import torch
 
 from oracle import sst_oracle as O
-
-REF = "/root/reference"
 
 
 def test_registry_builds_flagship_and_deepcopies_lists():
@@ -60,22 +57,20 @@ def test_lazy_dict_materialises_once():
     assert len(calls) == 1
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference configs not present")
 def test_reference_configs_load_and_build_unchanged():
-    """configs/sst (v1 names), configs/sst_refactor, configs/fsd and configs/fsdv2 parse with the stand-in Config loader and every hot-path module
-    they name builds from the unmodified dict (SURVEY 8b)."""
+    """The model dicts of configs/sst (v1 names), configs/sst_refactor, configs/fsd and configs/fsdv2 (the reference's files as parsed by the
+    stand-in Config loader, tests/golden/reference_configs.npz, `python -m oracle.make_golden pins`): every hot-path module they name builds
+    from the unmodified dict (SURVEY 8b)."""
+    import ast
+    import numpy as np
     from sst_b200 import registry
-    from sst_b200.config import Config, find_hot_path_modules
-    files = sorted(glob.glob(f"{REF}/configs/sst/*.py") + glob.glob(f"{REF}/configs/sst_refactor/*.py") +
-                   glob.glob(f"{REF}/configs/fsd/*.py") + glob.glob(f"{REF}/configs/fsdv2/*.py"))
-    # configs/sst/to_be_done_do_not_use.py inherits from a _base_ file that does not exist in the reference tree: it cannot be
-    # loaded by mmcv either
-    files = [f for f in files if not f.endswith("to_be_done_do_not_use.py")]
-    assert len(files) >= 11 and sum("/configs/sst/" in f for f in files) >= 5
+    from sst_b200.config import find_hot_path_modules
+    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_configs.npz"))
+    files, models = [str(f) for f in z["files"]], [ast.literal_eval(str(m)) for m in z["models"]]
+    assert len(files) >= 11 and sum(f.startswith("configs/sst/") for f in files) >= 5
     built = {}
-    for f in files:
-        cfg = Config.fromfile(f)
-        for path, node in find_hot_path_modules(cfg.get("model", {}), registry.MODELS):
+    for f, model in zip(files, models):
+        for path, node in find_hot_path_modules(model, registry.MODELS):
             try:
                 m = registry.MODELS.build(node)
             except NotImplementedError as e:   # declared gaps (e.g. fusion layers) must be explicit
@@ -88,6 +83,34 @@ def test_reference_configs_load_and_build_unchanged():
               "SimpleSparseUNet", "VirtualVoxelMixer"):
         assert built.get(t, 0) >= 1, f"no config exercised {t}: {built}"
     assert not built.get("unsupported"), built.get("unsupported")
+
+
+def test_config_loader_base_chain_and_delete(tmp_path):
+    """Config.fromfile resolves a two-level `_base_` chain (list and string forms, relative paths), merges nested dicts key by key,
+    replaces a dict marked `_delete_=True`, and keeps what the leaf file defines last."""
+    from sst_b200.config import Config
+    (tmp_path / "_base_").mkdir()
+    (tmp_path / "_base_" / "model.py").write_text(
+        "voxel_size = (0.32, 0.32, 6)\n"
+        "model = dict(type='DynamicVoxelNet', voxel_encoder=dict(type='DynamicVFE', in_channels=3, feat_channels=[64, 128]),\n"
+        "             backbone=dict(type='SSTv2', d_model=[128] * 6, nhead=[8] * 6, num_blocks=6))\n")
+    (tmp_path / "mid.py").write_text(
+        "_base_ = ['./_base_/model.py']\n"
+        "model = dict(backbone=dict(num_blocks=2), neck=dict(type='SECONDFPN', in_channels=[128]))\n")
+    (tmp_path / "leaf.py").write_text(
+        "_base_ = './mid.py'\n"
+        "import math\n"
+        "voxel_size = (0.25, 0.25, 0.2)\n"
+        "model = dict(voxel_encoder=dict(feat_channels=[32, 32]), neck=dict(_delete_=True, type='Voxel2PointScatterNeck'))\n")
+    cfg = Config.fromfile(str(tmp_path / "leaf.py"))
+    assert cfg["voxel_size"] == (0.25, 0.25, 0.2) and "math" not in cfg and "_base_" not in cfg
+    m = cfg.model
+    assert m.type == "DynamicVoxelNet"
+    assert m["voxel_encoder"] == dict(type='DynamicVFE', in_channels=3, feat_channels=[32, 32])
+    assert m["backbone"] == dict(type='SSTv2', d_model=[128] * 6, nhead=[8] * 6, num_blocks=2)
+    assert m["neck"] == dict(type='Voxel2PointScatterNeck')
+    with pytest.raises(AttributeError):
+        m.no_such_key
 
 
 def test_product_synth_frame_equals_oracle_generator():

@@ -1,53 +1,37 @@
-"""CPU, build container only: oracle/fsd_oracle.py (FSD instance grouping, SURVEY 8f next-3) against the reference's own functions and
-ClusterAssigner class compiled from mmdet3d/models/detectors/single_stage_fsd.py (unmodified source, oracle/ref_shim.reference_functions)."""
+"""CPU: oracle/fsd_oracle.py (FSD instance grouping, SURVEY 8f next-3) against what the reference's own functions and ClusterAssigner class
+(compiled from mmdet3d/models/detectors/single_stage_fsd.py, unmodified source, by oracle/ref_shim.reference_functions) returned on the
+same seeded inputs - recorded bit-exactly in tests/golden/ref_fsd_pins.npz by `python -m oracle.make_golden pins`."""
+import os
+
 import pytest
 import torch
 
-from oracle import fsd_oracle as FO, ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
-FSD = "mmdet3d/models/detectors/single_stage_fsd.py"
+from oracle import fsd_oracle as FO, golden_io as GI, make_golden as MG
 
 
 @pytest.fixture(scope="module")
-def RF():
-    return ref_shim.reference_functions(FSD, ["filter_almost_empty", "find_connected_componets", "find_connected_componets_single_batch",
-                                              "modify_cluster_by_class", "ClusterAssigner"])
+def Z():
+    return GI.load(os.path.join(os.path.dirname(__file__), "golden", "ref_fsd_pins.npz"))
 
 
 @pytest.mark.parametrize("dist", [0.1, 0.6, 2.0])
-def test_connected_components_match_reference(RF, dist):
+def test_connected_components_match_reference(Z, dist):
     pts, bidx = FO.synth_centres(3, 3, 700)
-    ref = RF["find_connected_componets"](pts, bidx, dist)
-    assert torch.equal(FO.find_connected_components(pts, bidx, dist), ref)
-    assert torch.equal(FO.connected_components_large(pts, bidx, dist), ref)
-    one = RF["find_connected_componets_single_batch"](pts[:700], bidx[:700], dist)
-    assert torch.equal(FO.find_connected_components(pts[:700], torch.zeros(700, dtype=torch.int32), dist), one)
+    GI.check(Z, f"cc.{dist}", FO.find_connected_components(pts, bidx, dist))
+    GI.check(Z, f"cc.{dist}", FO.connected_components_large(pts, bidx, dist))
+    GI.check(Z, f"cc_single.{dist}", FO.find_connected_components(pts[:700], torch.zeros(700, dtype=torch.int32), dist))
 
 
-def test_cluster_assigner_matches_reference(RF):
-    cfg = dict(cluster_voxel_size=dict(Car=(0.3, 0.3, 6), Cyclist=(0.2, 0.2, 6), Pedestrian=(0.05, 0.05, 6)), min_points=2,
-               point_cloud_range=[-80, -80, -2, 80, 80, 4], connected_dist=dict(Car=0.6, Cyclist=0.4, Pedestrian=0.1),
-               class_names=['Car', 'Cyclist', 'Pedestrian'])
-    ca = RF["ClusterAssigner"](**cfg)
-    ca.num_classes = 3
-    ca.train()   # the batched scipy branch (single_stage_fsd.py:984-985)
-    pts_l, b_l = [], []
-    for i, blob in enumerate((0.5, 0.3, 0.08)):
-        p, b = FO.synth_centres(10 + i, 2, 1500, blob=blob)
-        order = torch.argsort(b, stable=True)
-        pts_l.append(p[order])
-        b_l.append(b[order])
-    inds, masks = ca(pts_l, b_l, origin_points=[None] * 3)
+def test_cluster_assigner_matches_reference(Z):
+    cfg = MG.FSD_CA_CFG
+    pts_l, b_l = MG.pin_cluster_inputs()   # the batched scipy branch of ClusterAssigner in train() (single_stage_fsd.py:984-985)
     for i, name in enumerate(cfg["class_names"]):
         o_inds, o_mask = FO.cluster_assigner_single_class(pts_l[i], b_l[i], cfg["cluster_voxel_size"][name], 2, cfg["point_cloud_range"],
                                                           cfg["connected_dist"][name])
-        assert torch.equal(o_mask, masks[i])
-        assert torch.equal(inds[i][:, 0], torch.full_like(inds[i][:, 0], i))
-        assert torch.equal(o_inds, inds[i][:, 1:].int())
-    ca.eval()    # eval branch: find_connected_componets_single_batch on a one-sample batch
-    m0 = b_l[0] == 0
-    inds1, _ = ca([pts_l[0][m0]], [b_l[0][m0]], origin_points=[None])
+        GI.check(Z, f"ca.mask{i}", o_mask)
+        GI.check(Z, f"ca.class{i}", torch.full((o_inds.shape[0],), i, dtype=torch.long))
+        GI.check(Z, f"ca.inds{i}", o_inds.int())
+    m0 = b_l[0] == 0   # eval branch: find_connected_componets_single_batch on a one-sample batch
     o_inds, _ = FO.cluster_assigner_single_class(pts_l[0][m0], b_l[0][m0], cfg["cluster_voxel_size"]["Car"], 2, cfg["point_cloud_range"], 0.6,
                                                  single_batch=True)
-    assert torch.equal(o_inds, inds1[0][:, 1:].int())
+    GI.check(Z, "ca.eval_inds", o_inds.int())

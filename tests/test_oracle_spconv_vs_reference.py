@@ -1,19 +1,18 @@
-"""CPU, build container only: pins oracle/spconv_oracle.py (dense restatement of the sparse convolutions, SURVEY 8f next-1) against the
-reference's own vendored spconv v1 - its Python layers imported unmodified through oracle/ref_shim.load_spconv(), its C++ sources
-compiled unmodified into oracle/_ref by oracle/build_ref.py - and against the reference's SimpleSparseUNet / VirtualVoxelMixer classes.
-Skipped where /root/reference does not exist (the GPU box): there tests/golden/spconv_*.npz carry the reference's outputs."""
+"""CPU: pins oracle/spconv_oracle.py (dense restatement of the sparse convolutions, SURVEY 8f next-1) against the reference's own vendored
+spconv v1 - its Python layers imported unmodified through oracle/ref_shim.load_spconv(), its C++ sources compiled unmodified by
+oracle/build_ref.py - and its SimpleSparseUNet / VirtualVoxelMixer classes, run with seeded weights on seeded inputs.  What the reference
+returned is recorded in tests/golden/ref_spconv_pins.npz by `python -m oracle.make_golden pins`."""
+import os
+
 import pytest
 import torch
 
-from oracle import build_ref, ref_shim, spconv_oracle as SO
-
-pytestmark = pytest.mark.skipif(not ref_shim.available() or not build_ref.built("sparse_conv_ext_ref"),
-                                reason="reference tree / oracle/_ref spconv build not present")
+from oracle import golden_io as GI, make_golden as MG, spconv_oracle as SO
 
 
 @pytest.fixture(scope="module")
-def S():
-    return ref_shim.load_spconv()
+def Z():
+    return GI.load(os.path.join(os.path.dirname(__file__), "golden", "ref_spconv_pins.npz"))
 
 
 def _by_coor(feats, coors):
@@ -24,91 +23,62 @@ def _by_coor(feats, coors):
     return feats[order], coors[order]
 
 
-@pytest.mark.parametrize("ks,stride,padding", [(3, 2, 1), (3, 2, (0, 1, 1)), ((3, 1, 1), (2, 1, 1), 0), (2, 2, 0)])
-def test_sparse_conv_and_inverse_match_reference(S, ks, stride, padding):
+@pytest.mark.parametrize("ks,stride,padding", MG.SPCONV_PIN_CONV)
+def test_sparse_conv_and_inverse_match_reference(Z, ks, stride, padding):
+    case = MG.SPCONV_PIN_CONV.index((ks, stride, padding))
     feats, coors = SO.synth_sparse(1, 2, (9, 20, 24), 300, 8)
-    torch.manual_seed(0)
-    conv = S.SparseConv3d(8, 12, ks, stride=stride, padding=padding, bias=False, indice_key="k")
-    inv = S.SparseInverseConv3d(12, 6, ks, indice_key="k", bias=False)
-    x = S.SparseConvTensor(feats, coors, [9, 20, 24], 2)
-    with torch.no_grad():
-        y = conv(x)
-        z = inv(y)
-    of, oc, oshape = SO.sparse_conv(feats, coors, 2, [9, 20, 24], conv.weight.detach(), conv.stride, conv.padding)
-    assert list(y.spatial_shape) == oshape
-    yf, yc = _by_coor(y.features, y.indices)
-    assert torch.equal(yc.int(), oc)          # oracle order is lexicographic
-    torch.testing.assert_close(of, yf, rtol=1e-4, atol=1e-5)
+    ks, stride, padding = Z[f"conv{case}.geometry"]
+    w = GI.seeded_state([("weight", [*ks, 8, 12])], 200 + case)["weight"]
+    wi = GI.seeded_state([("weight", [*ks, 12, 6])], 210 + case)["weight"]
+    of, oc, oshape = SO.sparse_conv(feats, coors, 2, [9, 20, 24], w, stride, padding)
+    assert oshape == Z[f"conv{case}.spatial_shape"]
+    GI.check(Z, f"conv{case}.coors", oc)          # oracle order is lexicographic
+    GI.check(Z, f"conv{case}.out", of, rtol=1e-4, atol=1e-5)
     # the neighbour table regrouped from the reference's index pairs
-    nbr = SO.neighbour_table(coors, oc, 2, [9, 20, 24], conv.kernel_size, conv.stride, conv.padding)
-    torch.testing.assert_close(SO.indice_conv(feats, nbr, conv.weight.detach()), of, rtol=1e-4, atol=1e-5)
-    zi = SO.inverse_conv(of, oc, 2, oshape, coors, [9, 20, 24], inv.weight.detach(), conv.stride, conv.padding)
-    assert torch.equal(z.indices, coors)      # the inverse conv restores the couple conv's input rows, in order
-    torch.testing.assert_close(zi, z.features, rtol=1e-4, atol=1e-5)
+    nbr = SO.neighbour_table(coors, oc, 2, [9, 20, 24], ks, stride, padding)
+    torch.testing.assert_close(SO.indice_conv(feats, nbr, w), of, rtol=1e-4, atol=1e-5)
+    zi = SO.inverse_conv(of, oc, 2, oshape, coors, [9, 20, 24], wi, stride, padding)
+    GI.check(Z, f"conv{case}.inv_coors", coors)   # the inverse conv restores the couple conv's input rows, in order
+    GI.check(Z, f"conv{case}.inv_out", zi, rtol=1e-4, atol=1e-5)
 
 
-@pytest.mark.parametrize("ks,padding", [(3, 1), ((3, 1, 1), (1, 0, 0)), (3, 0), (3, (0, 1, 1))])
-def test_subm_conv_matches_reference(S, ks, padding):
+@pytest.mark.parametrize("ks,padding", MG.SPCONV_PIN_SUBM)
+def test_subm_conv_matches_reference(Z, ks, padding):
     """incl. layers built with padding != k//2: the index generation centres every SubM conv (spconv_ops.h:74-78)"""
+    case = MG.SPCONV_PIN_SUBM.index((ks, padding))
     feats, coors = SO.synth_sparse(2, 2, (7, 18, 18), 250, 8)
-    torch.manual_seed(1)
-    conv = S.SubMConv3d(8, 10, ks, padding=padding, bias=True, indice_key="s")
-    with torch.no_grad():
-        y = conv(S.SparseConvTensor(feats, coors, [7, 18, 18], 2))
-    assert torch.equal(y.indices, coors)
-    o = SO.subm_conv(feats, coors, 2, [7, 18, 18], conv.weight.detach(), conv.bias.detach())
-    torch.testing.assert_close(o, y.features, rtol=1e-4, atol=1e-5)
-    nbr = SO.neighbour_table(coors, coors, 2, [7, 18, 18], conv.kernel_size, [1, 1, 1], [k // 2 for k in conv.kernel_size])
-    torch.testing.assert_close(SO.indice_conv(feats, nbr, conv.weight.detach(), shift=conv.bias.detach()), y.features, rtol=1e-4, atol=1e-5)
+    ks = Z[f"subm{case}.kernel_size"]
+    wb = GI.seeded_state([("weight", [*ks, 8, 10]), ("bias", [10])], 220 + case)
+    GI.check(Z, f"subm{case}.coors", coors)
+    o = SO.subm_conv(feats, coors, 2, [7, 18, 18], wb["weight"], wb["bias"])
+    GI.check(Z, f"subm{case}.out", o, rtol=1e-4, atol=1e-5)
+    nbr = SO.neighbour_table(coors, coors, 2, [7, 18, 18], ks, [1, 1, 1], [k // 2 for k in ks])
+    GI.check(Z, f"subm{case}.out", SO.indice_conv(feats, nbr, wb["weight"], shift=wb["bias"]), rtol=1e-4, atol=1e-5)
 
 
-UNET = dict(in_channels=8, sparse_shape=[9, 32, 32], order=('conv', 'norm', 'act'), norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01),
-            base_channels=8, output_channels=16, encoder_channels=((8,), (8, 8, 8), (16, 16, 16), (16, 16, 16)),
-            encoder_paddings=((1,), (1, 1, 1), (1, 1, 1), ((0, 1, 1), 1, 1)),
-            decoder_channels=((16, 16, 16), (16, 16, 8), (8, 8, 8), (8, 8, 8)), decoder_paddings=((1, 1), (1, 0), (0, 0), (0, 1)))
-
-
-def _randomise_bn(m, seed):
-    g = torch.Generator().manual_seed(seed)
-    for mod in m.modules():
-        if isinstance(mod, torch.nn.BatchNorm1d):
-            mod.running_mean.copy_(torch.randn(mod.num_features, generator=g) * 0.2)
-            mod.running_var.copy_(torch.rand(mod.num_features, generator=g) + 0.5)
-            mod.weight.data.copy_(torch.rand(mod.num_features, generator=g) + 0.5)
-            mod.bias.data.copy_(torch.randn(mod.num_features, generator=g) * 0.2)
-
-
-def test_simple_sparse_unet_matches_reference(S):
-    torch.manual_seed(3)
-    net = S.SimpleSparseUNet(**UNET, return_multiscale_features=True).eval()
-    _randomise_bn(net, 5)
+def test_simple_sparse_unet_matches_reference(Z):
+    U = MG.SPCONV_PIN_UNET
+    sd = GI.seeded_state(Z["unet.spec"], 230)
     feats, coors = SO.synth_sparse(4, 2, (9, 32, 32), 500, 8)
-    with torch.no_grad():
-        out = net(dict(voxel_feats=feats, voxel_coors=coors))[0]
-    f, c, ms = SO.sparse_unet_forward(net.state_dict(), feats, coors, 2, UNET["sparse_shape"], UNET["encoder_channels"], UNET["encoder_paddings"],
-                                      UNET["decoder_channels"], UNET["decoder_paddings"], return_multiscale=True)
-    assert torch.equal(out["voxel_coors"], coors) and torch.equal(c, coors)
-    torch.testing.assert_close(f, out["voxel_feats"], rtol=1e-3, atol=1e-4)
-    assert len(ms) == len(out["decoder_features"]) == 4
-    for (mf, mc), ref in zip(ms, out["decoder_features"]):
-        rf, rc = _by_coor(ref.features, ref.indices)
+    f, c, ms = SO.sparse_unet_forward(sd, feats, coors, 2, U["sparse_shape"], U["encoder_channels"], U["encoder_paddings"],
+                                      U["decoder_channels"], U["decoder_paddings"], return_multiscale=True)
+    assert torch.equal(c, coors)
+    GI.check(Z, "unet.coors", coors)
+    GI.check(Z, "unet.out", f, rtol=1e-3, atol=1e-4)
+    assert len(ms) == Z["unet.n_levels"] == 4
+    for i, (mf, mc) in enumerate(ms):
         of, oc = _by_coor(mf, mc)
-        assert torch.equal(oc.int(), rc.int())
-        torch.testing.assert_close(of, rf, rtol=1e-3, atol=1e-4)
+        GI.check(Z, f"unet.ms{i}.coors", oc.int())
+        GI.check(Z, f"unet.ms{i}.out", of, rtol=1e-3, atol=1e-4)
 
 
-def test_virtual_voxel_mixer_matches_reference(S):
+def test_virtual_voxel_mixer_matches_reference(Z):
     """the mixer's conv_out is SubM kernel 3 / padding 0 on a fresh indice key - still a centred conv"""
-    cfg = dict(in_channels=8, sparse_shape=[8, 24, 24], norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01), base_channels=8,
-               output_channels=12, encoder_channels=((8,), (8, 8), (8, 8)), encoder_paddings=((1,), (1, 1), (1, 1)),
-               decoder_channels=((8, 8, 8), (8, 8, 8), (8, 8, 8)), decoder_paddings=((1, 1), (1, 1), (1, 1)))
-    torch.manual_seed(7)
-    net = S.VirtualVoxelMixer(**cfg).eval()
-    _randomise_bn(net, 9)
+    cfg = MG.SPCONV_PIN_MIXER
+    sd = GI.seeded_state(Z["mixer.spec"], 240)
     feats, coors = SO.synth_sparse(8, 3, (8, 24, 24), 300, 8)
-    with torch.no_grad():
-        rf, rc, rshape = net(feats, coors, 3)
-    f, c = SO.sparse_unet_forward(net.state_dict(), feats, coors, 3, cfg["sparse_shape"], cfg["encoder_channels"], cfg["encoder_paddings"],
+    f, c = SO.sparse_unet_forward(sd, feats, coors, 3, cfg["sparse_shape"], cfg["encoder_channels"], cfg["encoder_paddings"],
                                   cfg["decoder_channels"], cfg["decoder_paddings"], mixer_out=True)
-    assert torch.equal(rc, coors) and list(rshape) == cfg["sparse_shape"]
-    torch.testing.assert_close(f, rf, rtol=1e-3, atol=1e-4)
+    GI.check(Z, "mixer.coors", coors)
+    assert Z["mixer.spatial_shape"] == cfg["sparse_shape"]
+    GI.check(Z, "mixer.out", f, rtol=1e-3, atol=1e-4)

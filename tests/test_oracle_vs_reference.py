@@ -1,11 +1,11 @@
-"""CPU, build container only: runs the reference's own Python (unmodified, through oracle/ref_shim.py) beside the
-oracle on seeded inputs.  Skipped where /root/reference does not exist (e.g. the GPU box)."""
+"""CPU: pins the oracle to what the reference's own Python (unmodified, through oracle/ref_shim.py) computed on seeded inputs with seeded
+weights - outputs, gradients and state-dict layouts recorded in tests/golden/ref_sst_pins.npz by `python -m oracle.make_golden pins`."""
+import os
+
 import pytest
 import torch
 
-from oracle import ref_shim, sst_oracle as O
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+from oracle import golden_io as GI, make_golden as MG, sst_oracle as O
 
 VS = (0.32, 0.32, 6)
 RNG = [-74.88, -74.88, -2, 74.88, 74.88, 4]
@@ -14,147 +14,98 @@ DROP_TEST = {0: {'max_tokens': 30, 'drop_range': (0, 30)}, 1: {'max_tokens': 60,
 
 
 @pytest.fixture(scope="module")
-def R():
-    return ref_shim.load()
+def Z():
+    return GI.load(os.path.join(os.path.dirname(__file__), "golden", "ref_sst_pins.npz"))
 
 
-def test_config1_path(R):
+def test_config1_path(Z):
     """BASELINE config 1: 20k points, DynamicScatter + 1 SRA block d=64 h=4 on CPU (reference plumbing)."""
-    torch.manual_seed(0)
     pts = O.synth_frame(1000, 20000)
     coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0)
-    vfe = R.DynamicVFE(in_channels=3, feat_channels=[64, 64], with_cluster_center=True, with_voxel_center=True, voxel_size=VS,
-                       point_cloud_range=RNG, norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01)).eval()
-    il = R.SSTInputLayerV2(DROP_TEST, (12, 12, 1), (468, 468, 1), shuffle_voxels=False, debug=True, mute=True).eval()
-    bb = R.SSTv2(d_model=[64], nhead=[4], num_blocks=1, dim_feedforward=[128], output_shape=[468, 468], num_attached_conv=0,
-                 to_bev=False).eval()
-    with torch.no_grad():
-        vf_r, vc_r = vfe(pts, coors)
-        info_r = il(vf_r, vc_r, 1)
-        out_r = bb(info_r)[0]["voxel_feats"]
-    vf_o, vc_o = O.dynamic_vfe_forward(pts, coors, dict(vfe.state_dict()), VS, RNG, 2)
-    assert torch.equal(vc_o, vc_r)
-    torch.testing.assert_close(vf_o, vf_r, rtol=1e-6, atol=1e-6)
-    info_o = O.input_layer_v2(vf_r, vc_r, DROP_TEST, (12, 12, 1), (468, 468, 1))
+    wv, wb = GI.seeded_state(Z["config1.vfe_spec"], 101), GI.seeded_state(Z["config1.bb_spec"], 102)
+    vf_o, vc_o = O.dynamic_vfe_forward(pts, coors, wv, VS, RNG, 2)
+    GI.check(Z, "config1.vc", vc_o)
+    GI.check(Z, "config1.vf", vf_o, rtol=1e-6, atol=1e-6)
+    info_o = O.input_layer_v2(vf_o, vc_o, DROP_TEST, (12, 12, 1), (468, 468, 1))
     for i in range(2):
         for k in (f"batch_win_inds_shift{i}", f"coors_in_win_shift{i}", f"voxel_drop_level_shift{i}"):
-            assert torch.equal(info_r[k], info_o[k])
-    out_o = O.sstv2_forward(info_o, dict(bb.state_dict()), [4], 1)
-    torch.testing.assert_close(out_o, out_r, rtol=1e-5, atol=1e-6)
+            GI.check(Z, f"config1.{k}", info_o[k])
+    out_o = O.sstv2_forward(info_o, wb, [4], 1)
+    GI.check(Z, "config1.out", out_o, rtol=1e-5, atol=1e-6)
 
 
-def test_state_dict_keys_match_reference(R):
+def test_state_dict_keys_match_reference(Z):
     """The registered modules are checkpoint-compatible: same state-dict keys and shapes as the reference's."""
     from sst_b200 import flagship as fl
     cfg = fl.sst_cfg(num_blocks=2)
     vfe, il, bb = fl.build_sst(cfg)
-    r_vfe = R.DynamicVFE(**{k: v for k, v in cfg['voxel_encoder'].items() if k != 'type'})
-    r_bb = R.SSTv2(**{k: v for k, v in cfg['backbone'].items() if k != 'type'})
-    for ours, ref in ((vfe, r_vfe), (bb, r_bb)):
-        a = {k: tuple(v.shape) for k, v in ours.state_dict().items()}
-        b = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-        assert a == b
     from sst_b200.sst_modules import SSTv2
     lc = dict(cosine=True, non_shared_tau=True, use_bn=True)
     o = SSTv2(d_model=[32], nhead=[4], num_blocks=1, dim_feedforward=[64], num_attached_conv=0, to_bev=False, layer_cfg=lc)
-    r = R.SSTv2(d_model=[32], nhead=[4], num_blocks=1, dim_feedforward=[64], num_attached_conv=0, to_bev=False, layer_cfg=lc)
-    assert {k: tuple(v.shape) for k, v in o.state_dict().items()} == {k: tuple(v.shape) for k, v in r.state_dict().items()}
+    for name, ours in (("vfe", vfe), ("bb", bb), ("cosine", o)):
+        assert {k: list(v.shape) for k, v in ours.state_dict().items()} == Z[f"keys.{name}"], name
 
 
 @pytest.mark.parametrize("with_xyz,norm", [(True, False), (True, True), (False, False)])
-def test_voxel2point_neck(R, with_xyz, norm):
+def test_voxel2point_neck(Z, with_xyz, norm):
     """oracle.voxel2point_neck vs the unmodified reference Voxel2PointScatterNeck (necks/voxel2point_neck.py:28-62)."""
-    g = torch.Generator().manual_seed(5)
-    N, M, C = 5000, 700, 16
-    pts = O.synth_frame(3, N, extra_dims=1)
-    coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0).long()
-    vf = torch.randn(M, C, generator=g)
-    vf[::7] = -1.0  # dropped voxels are padded rows
-    inds = torch.randint(0, M, (N,), generator=g)
-    neck = R.Voxel2PointScatterNeck(point_cloud_range=RNG, voxel_size=VS, with_xyz=with_xyz, normalize_local_xyz=norm).eval()
-    r_out, r_mask = neck(pts, coors, vf, inds)
+    pts, coors, vf, inds = MG.pin_neck_inputs()
     o_out, o_mask = O.voxel2point_neck(pts, coors, vf, inds, VS, RNG, with_xyz, norm)
-    assert torch.equal(r_mask, o_mask) and torch.equal(r_out, o_out)
+    GI.check(Z, f"neck.{with_xyz}.{norm}.out", o_out)
+    GI.check(Z, f"neck.{with_xyz}.{norm}.mask", o_mask)
 
 
-def test_oracle_gradients_match_reference(R):
-    """The oracle is differentiable torch code, so autograd through it is the checker for the (round-2) backward kernels: pin it
-    now - parameter and input gradients of DynamicVFE -> SSTInputLayerV2 -> SSTv2 (eval-mode BN, one block) against the reference."""
-    torch.manual_seed(0)
+def test_oracle_gradients_match_reference(Z):
+    """The oracle is differentiable torch code, so autograd through it is the checker for the backward kernels: parameter and input
+    gradients of DynamicVFE -> SSTInputLayerV2 -> SSTv2 (eval-mode BN, one block) against the reference's autograd."""
     pts = O.synth_frame(1000, 6000)
     coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0)
-    vfe = R.DynamicVFE(in_channels=3, feat_channels=[32, 64], with_cluster_center=True, with_voxel_center=True, voxel_size=VS,
-                       point_cloud_range=RNG, norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01)).eval()
-    il = R.SSTInputLayerV2(DROP_TEST, (12, 12, 1), (468, 468, 1), shuffle_voxels=False, debug=True, mute=True).eval()
-    bb = R.SSTv2(d_model=[64], nhead=[4], num_blocks=1, dim_feedforward=[128], output_shape=[468, 468], num_attached_conv=0,
-                 to_bev=False).eval()
-    p_r = pts.clone().requires_grad_(True)
-    vf_r, vc_r = vfe(p_r, coors)
-    out_r = bb(il(vf_r, vc_r, 1))[0]["voxel_feats"]
-    out_r.square().mean().backward()
-    g_ref = {"vfe." + k: v.grad.clone() for k, v in vfe.named_parameters()}
-    g_ref.update({"bb." + k: v.grad.clone() for k, v in bb.named_parameters()})
-
-    wv = {k: v.detach().clone().requires_grad_(v.dtype.is_floating_point and k in dict(vfe.named_parameters()))
-          for k, v in vfe.state_dict().items()}
-    wb = {k: v.detach().clone().requires_grad_(v.dtype.is_floating_point) for k, v in bb.state_dict().items()}
+    vfe_spec, bb_spec = Z["grad.vfe_spec"], Z["grad.bb_spec"]
+    wv = {k: v.requires_grad_("running" not in k) for k, v in GI.seeded_state(vfe_spec, 103).items()}
+    wb = {k: v.requires_grad_(True) for k, v in GI.seeded_state(bb_spec, 104).items()}
     p_o = pts.clone().requires_grad_(True)
     vf_o, vc_o = O.dynamic_vfe_forward(p_o, coors, wv, VS, RNG, 2)
     info_o = O.input_layer_v2(vf_o, vc_o, DROP_TEST, (12, 12, 1), (468, 468, 1))
     out_o = O.sstv2_forward(info_o, wb, [4], 1)
     out_o.square().mean().backward()
-    torch.testing.assert_close(p_o.grad, p_r.grad, rtol=1e-4, atol=1e-7)
-    for k, g in g_ref.items():
+    GI.check(Z, "grad.points", p_o.grad, rtol=1e-4, atol=1e-7)
+    names = [k[len("grad."):] for k in Z["meta"] if k.startswith(("grad.vfe.", "grad.bb."))]
+    assert names
+    for k in names:
         w = wv[k[4:]] if k.startswith("vfe.") else wb[k[3:]]
-        torch.testing.assert_close(w.grad, g, rtol=2e-4, atol=1e-7, msg=k)
+        GI.check(Z, "grad." + k, w.grad, rtol=2e-4, atol=1e-7)
 
 
-def test_oracle_sir_gradients_match_reference(R):
+def test_oracle_sir_gradients_match_reference(Z):
     """Same for FSD's SIR (point-group MLP + pooling): oracle autograd == reference autograd."""
-    torch.manual_seed(1)
-    N, G = 3000, 40
-    g = torch.Generator().manual_seed(2)
-    points = torch.cat([torch.randn(N, 3, generator=g) * 10, torch.rand(N, 2, generator=g)], 1)
-    feats = torch.randn(N, 27, generator=g)
-    gid = torch.randint(0, G, (N,), generator=g)
-    coors = torch.stack([gid % 3, torch.zeros_like(gid), gid], 1)
-    fcl = torch.randn(N, 3, generator=g) * 2
-    # distinct inner lists: the reference's SIRLayer appends in_channels to rel_mlp_hidden_dims in place (voxel_encoder.py:665)
-    m = R.SIR(num_blocks=2, in_channels=[32, 37], feat_channels=[[32, 32], [32, 32]], rel_mlp_hidden_dims=[[16, 32], [16, 32]],
-              norm_cfg=dict(type='LN', eps=1e-3), mode='max', xyz_normalizer=[20, 20, 4], act='gelu', unique_once=True).eval()
-    f_r = feats.clone().requires_grad_(True)
-    a, b, _ = m(points, f_r, coors, fcl)
-    (a.square().mean() + b.square().mean()).backward()
-    w = {k: v.detach().clone().requires_grad_(True) for k, v in m.state_dict().items()}
+    points, feats, coors, fcl = MG.pin_sir_inputs()
+    w = {k: v.requires_grad_(True) for k, v in GI.seeded_state(Z["sir.spec"], 105).items()}
     f_o = feats.clone().requires_grad_(True)
     ao, bo, _ = O.sir_forward(points, f_o, coors, fcl, w, 2, 3, 2, [20, 20, 4])
     (ao.square().mean() + bo.square().mean()).backward()
-    torch.testing.assert_close(f_o.grad, f_r.grad, rtol=1e-4, atol=1e-7)
-    for k, p in m.named_parameters():
-        torch.testing.assert_close(w[k].grad, p.grad, rtol=2e-4, atol=1e-7, msg=k)
+    GI.check(Z, "sir.feats", f_o.grad, rtol=1e-4, atol=1e-7)
+    names = [k for k in w if "sir." + k in Z["meta"]]
+    assert len(names) == len(w), f"parameters without a reference record: {sorted(set(w) - set(names))}"
+    for k in names:
+        GI.check(Z, "sir." + k, w[k].grad, rtol=2e-4, atol=1e-7)
 
 
-def test_training_mode_vfe_matches_reference(R):
-    """Config-4 groundwork: DynamicVFE in TRAIN mode (naiveSyncBN1d batch statistics, single process) - outputs, input / parameter
-    gradients and the running-buffer update of one step against the reference."""
-    torch.manual_seed(0)
+def test_training_mode_vfe_matches_reference(Z):
+    """DynamicVFE in TRAIN mode (naiveSyncBN1d batch statistics, single process) - outputs, input / parameter gradients and the
+    running-buffer update of one step against the reference."""
     pts = O.synth_frame(1000, 6000)
     coors = torch.nn.functional.pad(O.dynamic_voxelize(pts, VS, RNG), (1, 0), value=0)
-    vfe = R.DynamicVFE(in_channels=3, feat_channels=[32, 64], with_cluster_center=True, with_voxel_center=True, voxel_size=VS,
-                       point_cloud_range=RNG, norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01)).train()
-    w0 = {k: v.detach().clone() for k, v in vfe.state_dict().items()}
-    p_r = pts.clone().requires_grad_(True)
-    vf_r, vc_r = vfe(p_r, coors)
-    vf_r.square().mean().backward()
-    w = {k: v.clone().requires_grad_(v.dtype.is_floating_point and "running" not in k) for k, v in w0.items()}
+    w0 = GI.seeded_state(Z["train.spec"], 106)
+    w = {k: v.clone().requires_grad_("running" not in k) for k, v in w0.items()}
     p_o = pts.clone().requires_grad_(True)
     vf_o, vc_o = O.dynamic_vfe_forward(p_o, coors, w, VS, RNG, 2, training=True)
     vf_o.square().mean().backward()
-    assert torch.equal(vc_o, vc_r)
-    torch.testing.assert_close(vf_o, vf_r, rtol=1e-5, atol=1e-6)
-    torch.testing.assert_close(p_o.grad, p_r.grad, rtol=1e-4, atol=1e-7)
-    for k, p in vfe.named_parameters():
-        torch.testing.assert_close(w[k].grad, p.grad, rtol=2e-4, atol=1e-7, msg=k)
+    GI.check(Z, "train.vc", vc_o)
+    GI.check(Z, "train.vf", vf_o, rtol=1e-5, atol=1e-6)
+    GI.check(Z, "train.points", p_o.grad, rtol=1e-4, atol=1e-7)
+    for k in w:
+        if "running" not in k:
+            GI.check(Z, "train." + k, w[k].grad, rtol=2e-4, atol=1e-7)
     # running buffers after the step (layer 0 sees the decorated points): nn.BatchNorm1d update with the unbiased variance
     with torch.no_grad():
         ls = [pts]
@@ -163,31 +114,24 @@ def test_training_mode_vfe_matches_reference(R):
         ls.append(O._center_offsets(pts, coors, VS, RNG))
         y0 = torch.nn.functional.linear(torch.cat(ls, 1), w0["vfe_layers.0.linear.weight"])
         rm, rv = O.bn_running_update(y0, w0["vfe_layers.0.norm.running_mean"], w0["vfe_layers.0.norm.running_var"], 0.01)
-    sd = vfe.state_dict()
-    torch.testing.assert_close(rm, sd["vfe_layers.0.norm.running_mean"], rtol=1e-5, atol=1e-7)
-    torch.testing.assert_close(rv, sd["vfe_layers.0.norm.running_var"], rtol=1e-5, atol=1e-7)
+    GI.check(Z, "train.vfe_layers.0.norm.running_mean", rm, rtol=1e-5, atol=1e-7)
+    GI.check(Z, "train.vfe_layers.0.norm.running_var", rv, rtol=1e-5, atol=1e-7)
 
 
-def test_dynamic_scatter_vfe_training_mode_matches_reference(R):
+def test_dynamic_scatter_vfe_training_mode_matches_reference(Z):
     """DynamicScatterVFE in train() (batch-statistics BatchNorm, autograd through scatter_v2): outputs and gradients of the oracle's
     training=True restatement against the reference class - the checker of the product's training composition"""
-    vs, rng = (0.25, 0.25, 0.2), [-80, -80, -2, 80, 80, 4]
-    torch.manual_seed(0)
-    m = R.DynamicScatterVFE(in_channels=5, feat_channels=[32, 32], with_cluster_center=True, with_voxel_center=True, voxel_size=vs,
-                            point_cloud_range=rng, norm_cfg=dict(type='naiveSyncBN1d', eps=1e-3, momentum=0.01), unique_once=True,
-                            rel_dist_scaler=10.0).train()
-    pts = torch.cat([torch.cat([O.synth_frame(3 + b, 3000), torch.rand(3000, 2)], 1) for b in range(2)])
-    co = torch.cat([torch.nn.functional.pad(O.dynamic_voxelize(pts[b * 3000:(b + 1) * 3000], vs, rng), (1, 0), value=b) for b in range(2)]).long()
-    x = pts.clone().requires_grad_(True)
-    vf, vc, inv = m(x, co, return_inv=True)
-    probe = torch.randn(vf.shape, generator=torch.Generator().manual_seed(1))
-    (vf * probe).sum().backward()
-    w = {k: v.detach().clone().requires_grad_(v.dtype.is_floating_point and "running" not in k) for k, v in m.state_dict().items()}
+    pts, co, vs, rng = MG.pin_dsvfe_points()
+    w = {k: v.requires_grad_("running" not in k) for k, v in GI.seeded_state(Z["dsvfe.spec"], 107).items()}
     x2 = pts.clone().requires_grad_(True)
     of, oc, oinv = O.dynamic_scatter_vfe_forward(x2, co, w, vs, rng, 2, rel_dist_scaler=10.0, training=True)
-    assert torch.equal(oc, vc) and torch.equal(oinv, inv)
-    torch.testing.assert_close(of, vf, rtol=1e-4, atol=1e-5)
+    GI.check(Z, "dsvfe.vc", oc)
+    GI.check(Z, "dsvfe.inv", oinv)
+    GI.check(Z, "dsvfe.vf", of, rtol=1e-4, atol=1e-5)
+    probe = torch.randn(of.shape, generator=torch.Generator().manual_seed(1))
     (of * probe).sum().backward()
-    torch.testing.assert_close(x2.grad, x.grad, rtol=1e-3, atol=1e-5)
-    for name, p in m.named_parameters():
-        torch.testing.assert_close(w[name].grad, p.grad, rtol=1e-3, atol=1e-4 * float(p.grad.abs().max()) + 1e-7)
+    GI.check(Z, "dsvfe.points", x2.grad, rtol=1e-3, atol=1e-5)
+    names = [k for k in w if "running" not in k]
+    assert names and all("dsvfe." + k in Z["meta"] for k in names), "parameters without a reference record"
+    for k in names:
+        GI.check(Z, "dsvfe." + k, w[k].grad, rtol=1e-3, atol=1e-4 * Z["meta"]["dsvfe." + k]["abs_max"] + 1e-7)

@@ -1,19 +1,34 @@
-"""The reference's OWN compiled voxel_layer (oracle/_ref/voxel_layer_ref.so: /root/reference/mmdet3d/ops/voxel/src/*.cpp,*.cu
-built unmodified for sm_100a by oracle/build_ref.py) as the checker:
+"""The reference's OWN voxel_layer (mmdet3d/ops/voxel/src/*.cpp,*.cu, compiled unmodified for sm_100a by oracle/build_ref.py) as the
+checker, through what it returned on seeded inputs (tests/golden/ref_voxel_layer_pins.npz: its C++ on the CPU, `python -m oracle.make_golden
+pins`; tests/golden/ref_cuda_pins.npz: its CUDA kernels on a B200, `python -m oracle.make_golden cuda-pins`):
 
-  * CPU (not gpu): pins oracle.dynamic_voxelize to the reference C++ `dynamic_voxelize` (voxelization_cpu.cpp:7-41).
-  * GPU: libsstb200 vs the reference CUDA kernels on the same B200 - `dynamic_voxelize_gpu` (voxelization_cuda.cu:332-375)
-    and `dynamic_point_to_voxel_forward/backward_gpu` (scatter_points_cuda.cu:183-303); indices bit-exact.
+  * CPU (not gpu): pins oracle.dynamic_voxelize / hard_voxelize to the reference C++ (voxelization_cpu.cpp:7-142).
+  * GPU: libsstb200 vs the reference CUDA kernels - `dynamic_voxelize_gpu` (voxelization_cuda.cu:332-375) and
+    `dynamic_point_to_voxel_forward/backward_gpu` (scatter_points_cuda.cu:183-303); indices bit-exact.
 
-Skipped when the prebuilt extension is absent (it is git-ignored, travels with gpurun, and is rebuilt by
-__graft_entry__.build() wherever /root/reference exists)."""
+test_speed_vs_reference_cuda times the reference kernels themselves and runs only where oracle/_ref was built."""
+import os
+
 import pytest
 import torch
 
-from oracle import build_ref, sst_oracle as O
+from oracle import build_ref, golden_io as GI, make_golden as MG, sst_oracle as O
 
 VS = (0.32, 0.32, 6)
 RNG = [-74.88, -74.88, -2, 74.88, 74.88, 4]
+
+
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
+
+
+@pytest.fixture(scope="module")
+def Z():
+    return GI.load(os.path.join(GOLDEN, "ref_voxel_layer_pins.npz"))
+
+
+@pytest.fixture(scope="module")
+def ZC():
+    return GI.load(os.path.join(GOLDEN, "ref_cuda_pins.npz"))
 
 
 @pytest.fixture(scope="module")
@@ -27,54 +42,41 @@ def ref():
     return m
 
 
-@pytest.mark.parametrize("voxel_size,rng", [(VS, RNG), ((0.25, 0.25, 0.2), [-80, -80, -2, 80, 80, 4]),
-                                             ((0.1, 0.1, 0.15), [-51.2, -51.2, -5, 51.2, 51.2, 3])])
-def test_oracle_voxelize_equals_reference_cpp(ref, voxel_size, rng):
-    pts = O.synth_frame(11, 40000)
-    pts[::7, 0] += 200.0
-    pts[::11, 1] -= 300.0
-    co = torch.zeros((pts.shape[0], 3), dtype=torch.int32)
-    ref.dynamic_voxelize(pts, co, list(voxel_size), list(rng), 3)
-    assert torch.equal(co, O.dynamic_voxelize(pts, voxel_size, rng))
+@pytest.mark.parametrize("voxel_size,rng", MG.VOXEL_PIN_CASES)
+def test_oracle_voxelize_equals_reference_cpp(Z, voxel_size, rng):
+    case = MG.VOXEL_PIN_CASES.index((voxel_size, rng))
+    GI.check(Z, f"dyn{case}.coors", O.dynamic_voxelize(MG.pin_voxel_points(), voxel_size, rng))
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("P", [1, 20000, 150000])
-def test_voxelize_vs_reference_cuda(cuda, ref, P):
+@pytest.mark.parametrize("P", MG.VOXEL_CUDA_PIN_SIZES)
+def test_voxelize_vs_reference_cuda(cuda, ZC, P):
     from sst_b200 import ops
-    pts = O.synth_frame(77 + P, P).to(cuda)
-    pts[::5, 0] += 300.0
-    r = torch.zeros((P, 3), dtype=torch.int32, device=cuda)
-    ref.dynamic_voxelize(pts, r, list(VS), list(RNG), 3)
+    pts = MG.pin_voxel_cuda_points(P).to(cuda)
     g = torch.zeros((P, 3), dtype=torch.int32, device=cuda)
     ops.dynamic_voxelize(pts, g, VS, RNG, 3)
-    assert torch.equal(r, g)
+    GI.check(ZC, f"voxelize{P}", g)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("reduce", ["max", "mean", "sum"])
-@pytest.mark.parametrize("P,C,lo", [(150000, 128, 0), (200000, 3, -1), (5000, 64, -1), (17, 5, 0)])
-def test_dynamic_scatter_vs_reference_cuda(cuda, ref, reduce, P, C, lo):
-    """Forward + backward against the reference CUDA op (sorted unique + atomics) on identical device tensors."""
+@pytest.mark.parametrize("P,C,lo", MG.SCATTER_PIN_CASES)
+def test_dynamic_scatter_vs_reference_cuda(cuda, ZC, reduce, P, C, lo):
+    """Forward + backward against what the reference CUDA op (sorted unique + atomics) returned for the same inputs on a B200."""
     from sst_b200 import ops
-    g = torch.Generator().manual_seed(P + C)
-    feats = (torch.rand(P, C, generator=g) * 100 - 50).to(cuda)
-    if P >= 100000:
-        coors = ops.Voxelization(VS, RNG, -1)(O.synth_frame(5, P).to(cuda))
-    else:
-        coors = torch.randint(lo, 20, (P, 3), generator=g, dtype=torch.int32).to(cuda)
-    r_f, r_c, r_m, r_n = ref.dynamic_point_to_voxel_forward(feats, coors, reduce)
+    feats, coors, g = MG.pin_scatter_inputs(P, C, lo)
+    feats, coors = feats.to(cuda), coors.to(cuda)
+    key = f"scatter.{reduce}.{P}.{C}"
     g_f, g_c, g_m, g_n = ops.dynamic_point_to_voxel_forward(feats, coors, reduce)
-    assert torch.equal(g_c, r_c) and torch.equal(g_m, r_m) and torch.equal(g_n, r_n)
-    if reduce == "max":
-        assert torch.equal(g_f, r_f)
-    else:  # the reference accumulates with fp32 atomics in arbitrary order
-        torch.testing.assert_close(g_f, r_f, rtol=1e-5, atol=2e-3 if reduce == "sum" else 1e-4)
-    grad = torch.randn(r_f.shape, generator=g).to(cuda)
-    r_g, g_g = torch.zeros_like(feats), torch.zeros_like(feats)
-    ref.dynamic_point_to_voxel_backward(r_g, grad, feats, r_f, r_m, r_n, reduce)
-    ops.dynamic_point_to_voxel_backward(g_g, grad, feats, r_f, r_m, r_n, reduce)
-    torch.testing.assert_close(g_g, r_g, rtol=1e-6, atol=1e-6)
+    GI.check(ZC, key + ".coors", g_c)
+    GI.check(ZC, key + ".map", g_m)
+    GI.check(ZC, key + ".count", g_n)
+    # the reference accumulates with fp32 atomics in arbitrary order
+    GI.check(ZC, key + ".feats", g_f, rtol=1e-5, atol=2e-3 if reduce == "sum" else 1e-4)
+    grad = torch.randn(g_f.shape, generator=g).to(cuda)
+    g_g = torch.zeros_like(feats)
+    ops.dynamic_point_to_voxel_backward(g_g, grad, feats, g_f, g_m, g_n, reduce)
+    GI.check(ZC, key + ".grad", g_g, rtol=1e-6, atol=1e-6)
 
 
 @pytest.mark.gpu
@@ -123,44 +125,26 @@ def test_speed_vs_reference_cuda(cuda, ref):
     assert out["dynamic_scatter_max_C128"]["speedup"] > 2.0 and out["dynamic_scatter_mean_C128"]["speedup"] > 2.0
 
 
-HV_CASES = [  # (P, F, voxel_size, range, max_points, max_voxels)
-    (20000, 4, (0.32, 0.32, 6), [-74.88, -74.88, -2, 74.88, 74.88, 4], 32, 20000),
-    (20000, 4, (0.32, 0.32, 6), [-74.88, -74.88, -2, 74.88, 74.88, 4], 5, 300),       # both caps bite
-    (30000, 5, (0.5, 0.5, 0.25), [-40, -40, -3, 40, 40, 1], 10, 16000),               # 3-D grid
-    (7, 3, (1.0, 1.0, 1.0), [0, 0, 0, 4, 4, 4], 2, 3),
-]
-
-
-def _hv_points(P, F):
-    pts = O.synth_frame(300 + P, P, extra_dims=F - 3)
-    pts[::13, 0] += 500.0  # out of range -> clamped by this fork's voxeliser
-    return pts
-
-
-@pytest.mark.parametrize("P,F,vs,rng,mp,mv", HV_CASES)
-def test_oracle_hard_voxelize_equals_reference_cpp(ref, P, F, vs, rng, mp, mv):
+@pytest.mark.parametrize("P,F,vs,rng,mp,mv", MG.HV_PIN_CASES[:-1])
+def test_oracle_hard_voxelize_equals_reference_cpp(Z, P, F, vs, rng, mp, mv):
     """Pins oracle.hard_voxelize to the reference's own `hard_voxelize_cpu` (voxelization_cpu.cpp:43-142)."""
-    pts = _hv_points(P, F)
-    voxels = torch.zeros((mv, mp, F))
-    coors = torch.zeros((mv, 3), dtype=torch.int32)
-    npts = torch.zeros((mv,), dtype=torch.int32)
-    n = ref.hard_voxelize(pts, voxels, coors, npts, list(vs), list(rng), mp, mv, 3)
-    ov, oc, on = O.hard_voxelize(pts, vs, rng, mp, mv)
-    assert n == ov.shape[0]
-    assert torch.equal(oc, coors[:n]) and torch.equal(on, npts[:n]) and torch.equal(ov, voxels[:n])
+    case = MG.HV_PIN_CASES.index((P, F, vs, rng, mp, mv))
+    ov, oc, on = O.hard_voxelize(MG.pin_hv_points(P, F), vs, rng, mp, mv)
+    assert ov.shape[0] == Z[f"hv{case}.n"]
+    GI.check(Z, f"hv{case}.coors", oc)
+    GI.check(Z, f"hv{case}.npts", on)
+    GI.check(Z, f"hv{case}.voxels", ov)
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("P,F,vs,rng,mp,mv", HV_CASES + [(150000, 4, (0.32, 0.32, 6), [-74.88, -74.88, -2, 74.88, 74.88, 4], 32, 32000)])
-def test_hard_voxelize_vs_reference(cuda, ref, P, F, vs, rng, mp, mv):
+@pytest.mark.parametrize("P,F,vs,rng,mp,mv", MG.HV_PIN_CASES)
+def test_hard_voxelize_vs_reference(cuda, Z, P, F, vs, rng, mp, mv):
     """libsstb200 `Voxelization(max_num_points > 0)` against the reference CPU implementation (bit-exact: pure data movement)."""
     from sst_b200 import ops
-    pts = _hv_points(P, F)
-    voxels = torch.zeros((mv, mp, F))
-    coors = torch.zeros((mv, 3), dtype=torch.int32)
-    npts = torch.zeros((mv,), dtype=torch.int32)
-    n = ref.hard_voxelize(pts, voxels, coors, npts, list(vs), list(rng), mp, mv, 3)
+    case = MG.HV_PIN_CASES.index((P, F, vs, rng, mp, mv))
     layer = ops.Voxelization(vs, rng, mp, mv).eval()
-    gv, gc, gn = layer(pts.to(cuda))
-    assert gv.shape[0] == n
-    assert torch.equal(gc.cpu(), coors[:n]) and torch.equal(gn.cpu(), npts[:n]) and torch.equal(gv.cpu(), voxels[:n])
+    gv, gc, gn = layer(MG.pin_hv_points(P, F).to(cuda))
+    assert gv.shape[0] == Z[f"hv{case}.n"]
+    GI.check(Z, f"hv{case}.coors", gc)
+    GI.check(Z, f"hv{case}.npts", gn)
+    GI.check(Z, f"hv{case}.voxels", gv)

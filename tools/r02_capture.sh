@@ -13,7 +13,7 @@ case $s in
 bench)
   # launch list (durations + DRAM bytes) of the bench command itself: the kernels of its first timed window (4 frames; the engines'
   # construction warm-ups run on empty buffers and are excluded by the profiler range bench.py opens under SSTB200_NCU_RANGE=1)
-  SSTB200_NCU_RANGE=1 SSTB200_BENCH_REPS=2 timeout 600 $NCU --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum \
+  SSTB200_NCU_RANGE=1 timeout 600 $NCU --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum \
       --profile-from-start off --csv --log-file $O/r02_launches_bench.csv \
       python bench.py --steps 4 --warmup 3 --no-train --no-fp32 --no-cpu-baseline > $O/r02_launches_bench.log 2>&1 ;;
 frame)
