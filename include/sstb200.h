@@ -240,6 +240,12 @@ int sstb200_dynamic_scatter_vfe_forward(sstb200_ctx* ctx, const sstb200_vfe_cfg*
                                         const int64_t* coors, int num_points, float* voxel_feats,
                                         int64_t* voxel_coors, int64_t* unq_inv, int32_t* num_voxels_dev,
                                         int32_t* num_voxels_host);
+/* DynamicScatterVFE over the rows of sstb200_voxelize_frames (the sync-free FSD segmentation engine): coors [num_points,4] int32
+ * (b,z,y,x), rows past the last frame (-1) belong to no voxel and get unq_inv -1; voxel_coors int32, unq_inv [num_points] int32.
+ * cfg->grid_zyx is the voxeliser's grid (every coordinate inside it); the voxel count is written to num_voxels_dev only. */
+int sstb200_dynamic_scatter_vfe_forward_i32(sstb200_ctx* ctx, const sstb200_vfe_cfg* cfg, const float* points, const int32_t* coors,
+                                            int num_points, float* voxel_feats, int32_t* voxel_coors, int32_t* unq_inv,
+                                            int32_t* num_voxels_dev);
 
 /* V1 (batched, sync-free form used by the frame engine): voxelise a batch of frames stored back to back.
  * points [capacity,F]; frame_offsets_dev: device int32 [num_frames+1] (row ranges of the frames, last entry =
@@ -333,6 +339,13 @@ int sstb200_voxel2point(sstb200_ctx* ctx, const float* points, int point_dims, c
                         int num_voxels, int channels, const int64_t* voxel2point_inds, int num_points, float padding,
                         const float voxel_size[3], const float pc_min[3], int with_xyz, int normalize_local_xyz, float* out,
                         uint8_t* mask_out, int32_t* num_out_dev, int32_t* num_out_host);
+/* N1' the same without a host sync: pts_coors [N,4] and voxel2point_inds [N] int32, num_points N = the point capacity, the voxel
+ * count read from num_voxels_dev; a point whose index is outside [0, voxel count) (e.g. -1: rows past the last frame) is not kept
+ * (mask 0).  The kept-row count is written to num_out_dev. */
+int sstb200_voxel2point_dev(sstb200_ctx* ctx, const float* points, int point_dims, const int32_t* pts_coors, const float* voxel_feats,
+                            const int32_t* num_voxels_dev, int channels, const int32_t* voxel2point_inds, int num_points, float padding,
+                            const float voxel_size[3], const float pc_min[3], int with_xyz, int normalize_local_xyz, float* out,
+                            uint8_t* mask_out, int32_t* num_out_dev);
 
 /* A4  the whole encoder stack (SSTv2.forward's block loop, mmdet3d/models/backbones/sst_v2.py:129-133 with
  * BasicShiftBlockV2.forward, models/sst/sst_basic_block_v2.py:144-169): layer l uses the windows of shift l % 2.
@@ -414,6 +427,28 @@ int sstb200_spconv_forward(sstb200_ctx* ctx, const float* feats, int c_in, const
  * chunks, so the last bits depend on the launch like the reference's backward. */
 int sstb200_spconv_backward_weight(sstb200_ctx* ctx, const float* feats, int c_in, const int32_t* nbr, int n_out, int kernel_volume,
                                    const float* grad_out, int c_out, float* grad_weight);
+
+/* Device-count variants of the three entry points above (capacity-sized buffers, one CUDA graph per frame): every row count is
+ * read from device memory (n_*_dev <= the capacity n_*_cap), nothing is read back to the host, and the kernels loop over the real
+ * rows with grids sized from the SM count.  Coordinates must lie inside batch_size / the shapes (not checked on the device).
+ * Rows of the outputs past the device count are left untouched.  Same tables and the same arithmetic as the host-count calls. */
+int sstb200_spconv_out_coors_dev(sstb200_ctx* ctx, const int32_t* in_coors, int n_in_cap, const int32_t* n_in_dev, int batch_size,
+                                 const int32_t in_shape[3], const int32_t out_shape[3], const int32_t ksize[3], const int32_t stride[3],
+                                 const int32_t padding[3], int32_t* out_coors, int out_cap, int32_t* num_out_dev);
+int sstb200_spconv_table_dev(sstb200_ctx* ctx, const int32_t* in_coors, int n_in_cap, const int32_t* n_in_dev, const int32_t* out_coors,
+                             int n_out_cap, const int32_t* n_out_dev, int batch_size, const int32_t in_shape[3], const int32_t out_shape[3],
+                             const int32_t ksize[3], const int32_t stride[3], const int32_t padding[3], int32_t* nbr, int32_t* nbr_inv);
+/* feats rows have pitch lda (floats), out rows ldo, residual rows ldr (all multiples of 4): a convolution can read one half of a
+ * wider matrix and write into one half of another (the decoder's [bottom || lateral] concatenation without a copy). */
+int sstb200_spconv_forward_dev(sstb200_ctx* ctx, const float* feats, int lda, int c_in, const int32_t* nbr, int n_out_cap,
+                               const int32_t* n_out_dev, int kernel_volume, const float* weight, const void* weight_h16, int c_out,
+                               const float* scale, const float* shift, const float* residual, int ldr, int relu, int precision, float* out,
+                               int ldo);
+/* SparseUNet.decoder_layer_forward's merge (mmdet3d/models/middle_encoders/sparse_unet.py reduce_channel + add):
+ * out[o, j] = x_merge[o, j] + sum_g cat[o, j * r + g], r = cat_channels / channels; x_merge / out [n, channels], cat [n, cat_channels],
+ * the group sum first, then the add (torch's order). */
+int sstb200_spconv_decoder_merge(sstb200_ctx* ctx, const float* x_merge, const float* cat, int channels, int cat_channels, int n_cap,
+                                 const int32_t* n_dev, float* out);
 
 /* ---- next-3 (SURVEY 8f): FSD instance grouping.  find_connected_componets / _single_batch / _gpu
  * (mmdet3d/models/detectors/single_stage_fsd.py:37-81; TorchEx connected_components at :20,39-45): two centres of the same sample are

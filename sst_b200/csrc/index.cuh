@@ -118,7 +118,10 @@ static void launch_mark_rows(sstb200_ctx* c, const TI* rows, int n, const Extent
     launch_pdl(mark_rows_kernel<TI, true>, dim3(grid), dim3(1024), smem, c->stream, rows, n, e, negative_is_invalid, k.keys, k.bitmap, k.flags,
                n_dev, (uint32_t)k.nwords);
   } else {
-    launch_pdl(mark_rows_kernel<TI, false>, dim3((n + 255) / 256), dim3(256), (size_t)0, c->stream, rows, n, e, negative_is_invalid, k.keys,
+    int grid = (n + 255) / 256;
+    if (n_dev && grid > c->num_sms * 8) grid = c->num_sms * 8;   // n is a capacity: the grid-stride loop covers the real rows
+    if (grid < 1) grid = 1;
+    launch_pdl(mark_rows_kernel<TI, false>, dim3(grid), dim3(256), (size_t)0, c->stream, rows, n, e, negative_is_invalid, k.keys,
                k.bitmap, k.flags, n_dev, 0u);
   }
 }

@@ -7,18 +7,23 @@
 #include <stdarg.h>
 #include "common.cuh"
 
-__global__ void __launch_bounds__(256) v2p_mask_kernel(const float* __restrict__ voxel_feats, int C, const long long* __restrict__ inds, int N,
-                                                       int M, float padding, uint32_t* __restrict__ keep, uint8_t* __restrict__ mask_out,
-                                                       int32_t* __restrict__ err) {
+// TI: index type of inds / coors (int64 from the modules, int32 from the sync-free engine).  M_dev != nullptr: the voxel count is
+// read from the device and an index outside [0, M) marks a point that is not kept (no voxel: rows past the last frame) instead
+// of an error.
+template <typename TI>
+__global__ void __launch_bounds__(256) v2p_mask_kernel(const float* __restrict__ voxel_feats, int C, const TI* __restrict__ inds, int N,
+                                                       int M, const int32_t* __restrict__ M_dev, float padding, uint32_t* __restrict__ keep,
+                                                       uint8_t* __restrict__ mask_out, int32_t* __restrict__ err) {
   pdl_wait();
   pdl_launch();
   const int lane = threadIdx.x & 31;
   const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (i >= N) return;
-  const long long v = inds[i];
+  if (M_dev) M = *M_dev;
+  const long long v = (long long)inds[i];
   if (v < 0 || v >= M) {
     if (lane == 0) {
-      *err = 1;
+      if (!M_dev) *err = 1;
       keep[i] = 0;
       mask_out[i] = 0;
     }
@@ -34,8 +39,9 @@ __global__ void __launch_bounds__(256) v2p_mask_kernel(const float* __restrict__
   }
 }
 
-__global__ void __launch_bounds__(256) v2p_write_kernel(const float* __restrict__ points, int Cp, const long long* __restrict__ coors,
-                                                        const float* __restrict__ voxel_feats, int C, const long long* __restrict__ inds, int N,
+template <typename TI>
+__global__ void __launch_bounds__(256) v2p_write_kernel(const float* __restrict__ points, int Cp, const TI* __restrict__ coors,
+                                                        const float* __restrict__ voxel_feats, int C, const TI* __restrict__ inds, int N,
                                                         const uint32_t* __restrict__ keep, const uint32_t* __restrict__ pos, float vx, float vy,
                                                         float vz, float x0, float y0, float z0, int with_xyz, int normalize,
                                                         float* __restrict__ out) {
@@ -45,7 +51,7 @@ __global__ void __launch_bounds__(256) v2p_write_kernel(const float* __restrict_
   const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (i >= N || !keep[i]) return;
   const int Co = C + (with_xyz ? 3 : 0);
-  const float* row = voxel_feats + (size_t)inds[i] * C;
+  const float* row = voxel_feats + (size_t)(long long)inds[i] * C;
   float* o = out + (size_t)pos[i] * Co;
   for (int c = lane; c < C; c += 32) o[c] = row[c];
   if (with_xyz && lane < 3) {
@@ -82,10 +88,10 @@ extern "C" int sstb200_voxel2point(sstb200_ctx* c, const float* points, int Cp, 
   CUDA_TRY(c, cudaMemsetAsync(z, 0, scan_temps_bytes(N), c->stream));
   int32_t* err = (int32_t*)(st.ticket + 2);
   const unsigned blocks = (unsigned)(((size_t)N * 32 + 255) / 256);
-  launch_pdl(v2p_mask_kernel, dim3(blocks), dim3(256), (size_t)0, c->stream, voxel_feats, C, (const long long*)voxel2point_inds, N, M, padding, keep,
-             mask_out, err);
+  launch_pdl(v2p_mask_kernel<long long>, dim3(blocks), dim3(256), (size_t)0, c->stream, voxel_feats, C, (const long long*)voxel2point_inds, N, M,
+             (const int32_t*)nullptr, padding, keep, mask_out, err);
   launch_exclusive_scan(c->stream, LoadU32{keep}, (size_t)N, nullptr, st, pos, st.ticket + 1, true);
-  launch_pdl(v2p_write_kernel, dim3(blocks), dim3(256), (size_t)0, c->stream, points, Cp, (const long long*)pts_coors, voxel_feats, C,
+  launch_pdl(v2p_write_kernel<long long>, dim3(blocks), dim3(256), (size_t)0, c->stream, points, Cp, (const long long*)pts_coors, voxel_feats, C,
              (const long long*)voxel2point_inds, N, (const uint32_t*)keep, (const uint32_t*)pos, voxel_size[0], voxel_size[1], voxel_size[2], pc_min[0],
              pc_min[1], pc_min[2], with_xyz, normalize_local_xyz, out);
   LAUNCH_CHECK(c);
@@ -95,5 +101,37 @@ extern "C" int sstb200_voxel2point(sstb200_ctx* c, const float* points, int Cp, 
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   if (c->pinned_i32[1]) return sstb_fail(c, SSTB_ERR_ARG, "voxel2point: voxel2point_inds out of range [0, %d)", M);
   if (num_out_host) *num_out_host = c->pinned_i32[0];
+  return SSTB_OK;
+}
+
+// Sync-free form (the FSD segmentation engine): int32 coordinates / indices, the voxel count on the device, the kept-row count
+// written to num_out_dev by the compaction scan itself.  Nothing is read back.
+extern "C" int sstb200_voxel2point_dev(sstb200_ctx* c, const float* points, int Cp, const int32_t* pts_coors, const float* voxel_feats,
+                                       const int32_t* num_voxels_dev, int C, const int32_t* voxel2point_inds, int N, float padding,
+                                       const float voxel_size[3], const float pc_min[3], int with_xyz, int normalize_local_xyz, float* out,
+                                       uint8_t* mask_out, int32_t* num_out_dev) {
+  CHECK_ARG(c, c && N >= 0 && C >= 1 && Cp >= 3 && num_out_dev);
+  if (N == 0) {
+    CUDA_TRY(c, cudaMemsetAsync(num_out_dev, 0, 4, c->stream));
+    return SSTB_OK;
+  }
+  CHECK_ARG(c, points && pts_coors && voxel_feats && num_voxels_dev && voxel2point_inds && out && mask_out && voxel_size && pc_min);
+  arena_reset(c);
+  int rc = arena_reserve(c, 2 * al256((size_t)N * 4 + 64) + scan_temps_bytes(N) + 4096);
+  if (rc) return rc;
+  uint32_t* keep = arena_alloc<uint32_t>(c, (size_t)N + 2);
+  uint32_t* pos = arena_alloc<uint32_t>(c, (size_t)N + 2);
+  uint8_t* z = arena_alloc<uint8_t>(c, scan_temps_bytes(N));
+  if (!keep || !pos || !z) return sstb_fail(c, SSTB_ERR_WORKSPACE, "voxel2point_dev: arena");
+  ScanTemps st{(uint32_t*)z, (unsigned long long*)z + 32};
+  CUDA_TRY(c, cudaMemsetAsync(z, 0, scan_temps_bytes(N), c->stream));
+  const unsigned blocks = (unsigned)(((size_t)N * 32 + 255) / 256);
+  launch_pdl(v2p_mask_kernel<int32_t>, dim3(blocks), dim3(256), (size_t)0, c->stream, voxel_feats, C, voxel2point_inds, N, 0, num_voxels_dev,
+             padding, keep, mask_out, (int32_t*)nullptr);
+  launch_exclusive_scan(c->stream, LoadU32{keep}, (size_t)N, nullptr, st, pos, (uint32_t*)num_out_dev, true);
+  launch_pdl(v2p_write_kernel<int32_t>, dim3(blocks), dim3(256), (size_t)0, c->stream, points, Cp, pts_coors, voxel_feats, C, voxel2point_inds, N,
+             (const uint32_t*)keep, (const uint32_t*)pos, voxel_size[0], voxel_size[1], voxel_size[2], pc_min[0], pc_min[1], pc_min[2], with_xyz,
+             normalize_local_xyz, out);
+  LAUNCH_CHECK(c);
   return SSTB_OK;
 }

@@ -932,3 +932,13 @@ extern "C" int sstb200_dynamic_scatter_vfe_forward(sstb200_ctx* c, const sstb200
   return vfe_forward_impl<long long>(c, cfg, points, (const long long*)coors, P, voxel_feats, (long long*)voxel_coors,
                                      (long long*)unq_inv, num_dev, num_host);
 }
+
+// DynamicScatterVFE on the frame engine's rows: int32 (b,z,y,x) coordinates of sstb200_voxelize_frames (capacity rows; rows past the
+// last frame are -1 and belong to no voxel: their unq_inv is -1), int32 voxel coordinates and inverse, the voxel count on the device
+// only.  The grid (cfg->grid_zyx) comes from the voxeliser geometry.
+extern "C" int sstb200_dynamic_scatter_vfe_forward_i32(sstb200_ctx* c, const sstb200_vfe_cfg* cfg, const float* points, const int32_t* coors,
+                                                       int num_points, float* voxel_feats, int32_t* voxel_coors, int32_t* unq_inv,
+                                                       int32_t* num_voxels_dev) {
+  CHECK_ARG(c, unq_inv);
+  return vfe_forward_impl<int32_t>(c, cfg, points, coors, num_points, voxel_feats, voxel_coors, unq_inv, num_voxels_dev, nullptr);
+}

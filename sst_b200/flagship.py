@@ -145,3 +145,32 @@ def sir_bench(dev, reps=5, precisions=("bf16", "fp32")):
             ms = a.elapsed_time(b) / reps
             rec["bf16_tcgen05" if prec == "bf16" else "fp32_ffma"] = {"ms": ms, "tflops": flops / ms / 1e9}
     return rec
+
+
+# ---- the configs/fsd segmentation front (configs/fsd/fsd_waymoD1_1x.py:7-58): voxel encoder -> U-Net -> voxel-to-point neck ----------
+FSD_SEG_VOXEL_SIZE = (0.25, 0.25, 0.2)
+FSD_PC_RANGE = [-80, -80, -2, 80, 80, 4]
+FSD_VFE = dict(type="DynamicScatterVFE", in_channels=5, feat_channels=[64, 64], voxel_size=FSD_SEG_VOXEL_SIZE, with_cluster_center=True,
+               with_voxel_center=True, point_cloud_range=FSD_PC_RANGE, norm_cfg=dict(type="naiveSyncBN1d", eps=1e-3, momentum=0.01),
+               unique_once=True)
+FSD_NECK = dict(type="Voxel2PointScatterNeck", voxel_size=FSD_SEG_VOXEL_SIZE, point_cloud_range=FSD_PC_RANGE)
+
+
+def build_fsd_front(vfe_cfg=None, unet_cfg=None, neck_cfg=None, seed=0):
+    """(DynamicScatterVFE, SimpleSparseUNet, Voxel2PointScatterNeck) in eval mode, random init (torch.manual_seed(seed)) with the
+    BatchNorm statistics perturbed so that the folded scale / shift are not the identity."""
+    from . import neck_modules, spconv_modules  # noqa: F401  (registers the types)
+    from .registry import MODELS
+    torch.manual_seed(seed)
+    vfe = MODELS.build(dict(vfe_cfg or FSD_VFE)).eval()
+    unet = build_backbone(dict(unet_cfg or FSD_UNET)).eval()
+    neck = MODELS.build(dict(neck_cfg or FSD_NECK))
+    g = torch.Generator().manual_seed(seed + 1)
+    with torch.no_grad():
+        for m in list(vfe.modules()) + list(unet.modules()):
+            if isinstance(m, torch.nn.BatchNorm1d):
+                m.running_mean.copy_(torch.randn(m.num_features, generator=g) * 0.2)
+                m.running_var.copy_(torch.rand(m.num_features, generator=g) + 0.5)
+                m.weight.copy_(torch.rand(m.num_features, generator=g) + 0.5)
+                m.bias.copy_(torch.randn(m.num_features, generator=g) * 0.1)
+    return vfe, unet, neck

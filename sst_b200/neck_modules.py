@@ -16,6 +16,8 @@ NECKS = MODELS
 
 L.SIGNATURES["sstb200_voxel2point"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, L.vp, C.c_int, C.c_int, L.vp, C.c_int, C.c_float, L.P_f32,
                                                  L.P_f32, C.c_int, C.c_int, L.vp, L.vp, L.vp, L.P_i32])
+L.SIGNATURES["sstb200_voxel2point_dev"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, L.vp, L.vp, C.c_int, L.vp, C.c_int, C.c_float, L.P_f32,
+                                                     L.P_f32, C.c_int, C.c_int, L.vp, L.vp, L.vp])
 
 
 @NECKS.register_module()

@@ -35,6 +35,14 @@ L.SIGNATURES["sstb200_spconv_table"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, C.c
 L.SIGNATURES["sstb200_spconv_backward_weight"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, C.c_int, C.c_int, L.vp, C.c_int, L.vp])
 L.SIGNATURES["sstb200_spconv_forward"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, C.c_int, C.c_int, L.vp, L.vp, C.c_int, L.vp, L.vp, L.vp,
                                                    C.c_int, C.c_int, L.vp])
+# device-count variants (sync-free engines, sst_b200/fsd_engine.py)
+L.SIGNATURES["sstb200_spconv_out_coors_dev"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, C.c_int, L.P_i32, L.P_i32, L.P_i32, L.P_i32, L.P_i32,
+                                                         L.vp, C.c_int, L.vp])
+L.SIGNATURES["sstb200_spconv_table_dev"] = (C.c_int, [L.vp, L.vp, C.c_int, L.vp, L.vp, C.c_int, L.vp, C.c_int, L.P_i32, L.P_i32, L.P_i32,
+                                                     L.P_i32, L.P_i32, L.vp, L.vp])
+L.SIGNATURES["sstb200_spconv_forward_dev"] = (C.c_int, [L.vp, L.vp, C.c_int, C.c_int, L.vp, C.c_int, L.vp, C.c_int, L.vp, L.vp, C.c_int,
+                                                       L.vp, L.vp, L.vp, C.c_int, C.c_int, C.c_int, L.vp, C.c_int])
+L.SIGNATURES["sstb200_spconv_decoder_merge"] = (C.c_int, [L.vp, L.vp, L.vp, C.c_int, C.c_int, C.c_int, L.vp, L.vp])
 
 PREC = {"fp32": 0, "bf16": 1, "fp32_tc": 2}   # fp32_tc: fp32 tolerance on the tensor core (split-fp16 operands, 3 products per stage)
 

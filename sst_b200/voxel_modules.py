@@ -57,6 +57,8 @@ L.SIGNATURES["sstb200_dynamic_vfe_forward"] = (C.c_int, [L.vp, C.POINTER(_VfeCfg
                                                          L.vp, L.P_i32])
 L.SIGNATURES["sstb200_dynamic_scatter_vfe_forward"] = (C.c_int, [L.vp, C.POINTER(_VfeCfg), L.vp, L.vp, C.c_int, L.vp,
                                                                  L.vp, L.vp, L.vp, L.P_i32])
+L.SIGNATURES["sstb200_dynamic_scatter_vfe_forward_i32"] = (C.c_int, [L.vp, C.POINTER(_VfeCfg), L.vp, L.vp, C.c_int, L.vp, L.vp,
+                                                                     L.vp, L.vp])
 
 
 @VOXEL_ENCODERS.register_module()
